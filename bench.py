@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py -- Mpixels/s of the full multi-scale SSAO pipe (BASELINE.json metric), one JSON line.
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--workload 4k|1080p|8k|256]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--workload 4k|1080p|8k|256] [--dump-outputs DIR]
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N --master-addr 127.0.0.1 --master-port P \
         bench.py --gpus N --steps K --warmup W
 
@@ -23,6 +23,9 @@ frames -- weak scaling, no data-path collective (the reference keeps no temporal
             (configs[3]; speed-up against the one-GPU 8K time measured in the same run), batch of 64 x 1080p (configs[4])
 --impl reference: times that CPU restatement alone (the reference itself is HLSL + Unity C#, which cannot be built or run in
 this image: see DESIGN.md), all host threads, same workload / metric / config string.
+--dump-outputs DIR: after the timed steps, DIR/ao.npy (float32) holds the AO codes of the headline's last timed step (rank 0;
+            --impl reference: the oracle's last timed frame).  Inputs are generated deterministically, so two builds run with the
+            same arguments can be compared output for output.
 """
 from __future__ import annotations
 
@@ -47,6 +50,18 @@ WORKLOADS = {"256": (256, 256), "1080p": (1920, 1080), "4k": (3840, 2160), "8k":
 METRIC = "Mpixels/sec full SSAO pipe @4K"
 INTENSITY = 1.1   # Sponza.unity:969; every other parameter at the component default (AO.cs:20-52)
 BATCHES = 5       # timed batches of K steps; the median is the headline
+DUMP_BYTES = 64_000_000   # --dump-outputs budget
+
+
+def dump_output(dir_: str, name: str, a: np.ndarray) -> None:
+    """DIR/<name>.npy in float32.  An array above DUMP_BYTES is cut to a fixed sample of its flattened elements (the sorted
+    positions np.random.default_rng(0) picks), so dumps of the same workload still compare element for element."""
+    a = np.asarray(a, dtype=np.float32)
+    cap = DUMP_BYTES // 4 - 1024          # room for the .npy header
+    if a.size > cap:
+        a = a.reshape(-1)[np.sort(np.random.default_rng(0).choice(a.size, cap, replace=False))]
+    os.makedirs(dir_, exist_ok=True)
+    np.save(os.path.join(dir_, f"{name}.npy"), a)
 
 
 def workload_label(W: int, H: int) -> str:
@@ -175,14 +190,16 @@ def run_reference(args) -> None:
     from oracle.oracle import Oracle
     cores = pick_cpu_threads(W, H, depth)
     o = Oracle(W, H, threads=cores, intensity=INTENSITY)
-    # each step = one frame (a bounded sample of the workload: the same single frame every step); K and W as given
-    steps, warm = max(1, min(args.steps, 256)), max(0, min(args.warmup, 32))
+    # each step = one frame (the same single frame every step); exactly K timed steps
+    steps, warm = args.steps, max(0, min(args.warmup, 32))
     for _ in range(warm):
         o.run(depth)
     t0 = time.perf_counter()
     for _ in range(steps):
-        o.run(depth)
+        last = o.run(depth)
     dt = time.perf_counter() - t0
+    if args.dump_outputs:
+        dump_output(args.dump_outputs, "ao", last)
     v = W * H * steps / dt / 1e6
     line = {"impl": "reference", "metric": METRIC, "value": v, "unit": "Mpixels/s", "n_gpus": args.gpus, "steps": steps, "warmup": warm,
             "ms_per_step": dt / steps * 1e3, "higher_is_better": True, "scaling": "weak", "vs_baseline": None, "dtype": "f32",
@@ -213,7 +230,7 @@ def run_ours(args) -> None:
         dist.init_process_group("nccl", device_id=dev)
 
     W, H = WORKLOADS[args.workload]
-    K, Wm = max(1, args.steps), max(args.warmup, 3)
+    K, Wm = args.steps, max(args.warmup, 3)
     NBUF = 8
     S = max(1, args.streams)
     BAND_ONLY = args.only_8k
@@ -298,6 +315,8 @@ def run_ours(args) -> None:
         sampler.start()
         time.sleep(0.25)
     ms_med, ms_batches, aos, streams, submit = throughput(W, H, depths, outs, K)
+    # the last timed step wrote outs[(K - 1) % NBUF] (earlier steps on that buffer read the same depth frame)
+    last_ao = outs[(K - 1) % NBUF].cpu().numpy() if args.dump_outputs and rank == 0 else None
     ao = aos[0]
     launches = K * ao.kernels_per_frame
     t_end = time.time() + 0.6               # keep the load up a little longer so the 100 ms clock sampler sees it
@@ -486,6 +505,8 @@ def run_ours(args) -> None:
                         "d16_ingest": {"value": round(e2e_d16, 1), "h2d_bytes_per_step": W * H * 2, "note": "MEAO_DEPTH_RAW_D16_UNORM: the depth texture uploaded in its native 16-bit format"}},
                 "gpu_launches": int(launches), "clocks": clocks, "roofline": roofline, "kernels": kernels, "cpu_baseline": cpu,
                 "configs": configs, "rowtile": configs.get("8k_single_frame") if world > 1 else None, "composite": composite}
+        if last_ao is not None:
+            dump_output(args.dump_outputs, "ao", last_ao)
         print(json.dumps(line), flush=True)
     if world > 1:
         dist.destroy_process_group()
@@ -697,7 +718,12 @@ def main() -> None:
     ap.add_argument("--band-streams", type=int, default=12, help="band contexts per rank in the row-tiled 8K measurement")
     ap.add_argument("--only-8k", action="store_true", help="development aid: only the 8K single-frame / row-band measurement")
     ap.add_argument("--band-mode", default="native", choices=["native", "p2p"], help="halo exchange: peer stores inside the graph / NCCL send-recv between two graphs")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the AO of the last timed step as DIR/ao.npy (float32)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.only_8k:
+        ap.error("--dump-outputs covers the headline workload, which --only-8k skips")
     if args.impl == "reference":
         run_reference(args)
     else:
