@@ -54,6 +54,9 @@ namespace MiniEngineAO
         [DllImport(Lib)] public static extern int meao_resize(IntPtr ctx, int width, int height);
         [DllImport(Lib)] public static extern int meao_render(IntPtr ctx, IntPtr depthDev, int depthKind, IntPtr aoOutDev, IntPtr stream);
         [DllImport(Lib)] public static extern int meao_render_host(IntPtr ctx, float[] depth, int depthKind, byte[] aoOut);
+        [DllImport(Lib)] public static extern int meao_reserve_batch(IntPtr ctx, int frames);
+        [DllImport(Lib)] public static extern int meao_render_batch(IntPtr ctx, IntPtr depthDev, int depthKind, int frames, IntPtr aoOutDev, IntPtr stream);
+        [DllImport(Lib)] public static extern int meao_get_batch_buffer(IntPtr ctx, int frame, int bufferId, IntPtr hostOut, UIntPtr hostBytes);
         [DllImport(Lib)] public static extern int meao_bind_event(IntPtr ctx, int eventId, IntPtr depthDev, int depthKind, IntPtr aoOutDev, IntPtr stream);
         [DllImport(Lib)] public static extern IntPtr meao_get_render_event_func();
         [DllImport(Lib)] public static extern int meao_composite_framebuffer(IntPtr ctx, IntPtr aoDev, IntPtr colorDev, int colorFormat, IntPtr stream);
@@ -166,6 +169,13 @@ namespace MiniEngineAO
             // one plugin event replaces the ten DispatchCompute calls recorded by :511-531
             _renderCommand.IssuePluginEvent(MeaoNative.meao_get_render_event_func(), kEventId);
             _camera.AddCommandBuffer(CameraEvent.BeforeImageEffects, _renderCommand);          // :421
+        }
+
+        // Offline use (e.g. baking AO for a recorded depth sequence): `frames` camera-sized depth frames stacked tightly in device
+        // memory -> as many R8 AO frames, one graph replay.  Reserve the largest batch once, outside per-frame work.
+        public void RenderBatch(IntPtr depthDev, int depthKind, int frames, IntPtr aoOutDev, IntPtr stream)
+        {
+            MeaoNative.Check(_ctx, MeaoNative.meao_render_batch(_ctx, depthDev, depthKind, frames, aoOutDev, stream));
         }
 
         void OnDisable()

@@ -32,7 +32,8 @@ extern "C" {
 
 #define MEAO_ABI_VERSION 3   /* 2: + MeaoVariants, meao_stage_render_wide, meao_debug_view, meao_composite_debug, buffer ids 18..21
                               * 3: + MeaoVariants.single_scale, native peer halo exchange (meao_band_export / _connect / _step / _status),
-                              *      meao_bind_event takes the stream */
+                              *      meao_bind_event takes the stream;
+                              *      later (backward compatible): batched frames (meao_reserve_batch / meao_render_batch / meao_get_batch_buffer) */
 
 typedef struct MeaoCtx MeaoCtx;
 
@@ -162,6 +163,23 @@ int meao_render_host(MeaoCtx *ctx, const void *depth_host, int32_t depth_kind, u
  * (meao_host_alloc) for the copies to be asynchronous, and must stay valid until the matching wait. */
 int meao_render_host_async(MeaoCtx *ctx, const void *depth_host, int32_t depth_kind, uint8_t *ao_out_host, int32_t slot);
 int meao_host_wait(MeaoCtx *ctx, int32_t slot);
+
+/* ---- batched frames ---------------------------------------------------------------------------- */
+/* Batched frames: `frames` independent frames of the size set by meao_resize, stacked tightly:
+ * frame f of depth_dev starts at element f*W*H, frame f of ao_out_dev at byte f*W*H (R8).
+ * Every frame gives exactly what meao_render gives for it.  With graphs on, a batch is ONE graph replay (the DAG of a frame, every
+ * kernel covering all frames); MEAO_FLAG_NO_GRAPH issues the same launches directly.  Re-plans first if dirty, like meao_render.
+ * The intermediates of a batch live in a batch arena of their own: meao_get_buffer, meao_debug_view, the stage and band calls
+ * do not see a batch.  meao_resize and meao_destroy free it.
+ * meao_render_batch grows the arena on demand; growing is a synchronous allocation (device synchronise + cudaMalloc), so
+ * reserve the largest batch with meao_reserve_batch outside any timed region.
+ * MEAO_ERR_INVALID: frames < 1 or > 65535, NULL pointers, bad depth kind.  MEAO_ERR_UNSUPPORTED: a row band is set.
+ * MEAO_ERR_CUDA: plan-only context.  meao_launch_count grows by meao_kernels_per_frame per batch. */
+int meao_reserve_batch(MeaoCtx *ctx, int32_t frames);   /* allocate batch intermediates for >= frames (optional; render_batch grows on demand) */
+int meao_render_batch(MeaoCtx *ctx, const void *depth_dev, int32_t depth_kind, int32_t frames, void *ao_out_dev, void *stream);
+/* Buffer ids 1-16 and 18-21 of frame `frame` of the last batch, in the layout of meao_get_buffer (TiledDepth synthesised the
+ * same way; synchronises the device).  Id 17 is refused: the AO of a batch is in the caller's buffer. */
+int meao_get_batch_buffer(MeaoCtx *ctx, int32_t frame, int32_t buffer_id, void *host_out, size_t host_bytes);
 int meao_synchronize(MeaoCtx *ctx);
 void *meao_host_alloc(size_t bytes);                /* cudaHostAlloc; NULL on failure */
 void meao_host_free(void *p);

@@ -63,6 +63,9 @@ SIGNATURES = {
     "meao_render_host": (C.c_int, [C.c_void_p, C.c_void_p, C.c_int32, C.c_void_p]),
     "meao_render_host_async": (C.c_int, [C.c_void_p, C.c_void_p, C.c_int32, C.c_void_p, C.c_int32]),
     "meao_host_wait": (C.c_int, [C.c_void_p, C.c_int32]),
+    "meao_reserve_batch": (C.c_int, [C.c_void_p, C.c_int32]),
+    "meao_render_batch": (C.c_int, [C.c_void_p, C.c_void_p, C.c_int32, C.c_int32, C.c_void_p, C.c_void_p]),
+    "meao_get_batch_buffer": (C.c_int, [C.c_void_p, C.c_int32, C.c_int32, C.c_void_p, C.c_size_t]),
     "meao_synchronize": (C.c_int, [C.c_void_p]),
     "meao_host_alloc": (C.c_void_p, [C.c_size_t]),
     "meao_host_free": (None, [C.c_void_p]),

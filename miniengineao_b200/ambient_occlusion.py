@@ -184,6 +184,40 @@ class AmbientOcclusion:
         self._check(self._lib.meao_render(self._ctx, depth.data_ptr(), kind, out.data_ptr(), self._stream(stream)))
         return out
 
+    def render_batch(self, depth, out=None, *, linear: bool = False, stream=None):
+        """depth: contiguous CUDA tensor [B, H, W] of B independent frames, dtypes as in render().  Returns a CUDA uint8 tensor
+        [B, H, W]; frame b equals render(depth[b]).  One graph replay for the whole batch (meao_render_batch).  The first batch
+        larger than any before allocates the batch intermediates (synchronous): call reserve_batch(B) first to keep that out of
+        a timed loop."""
+        import torch
+        self.LateUpdate()
+        if not (depth.is_cuda and depth.is_contiguous()):
+            raise ValueError("depth must be a contiguous CUDA tensor")
+        if depth.dim() != 3 or tuple(depth.shape[1:]) != (self._height, self._width):
+            raise ValueError(f"depth shape {tuple(depth.shape)} != (B, {self._height}, {self._width})")
+        frames = int(depth.shape[0])
+        if out is None:
+            out = torch.empty((frames, self._height, self._width), dtype=torch.uint8, device=depth.device)
+        elif not (out.is_cuda and out.is_contiguous() and out.dtype == torch.uint8 and tuple(out.shape) == tuple(depth.shape)):
+            raise ValueError("out must be a contiguous CUDA uint8 tensor of the depth's shape")
+        kind = self._kind(str(depth.dtype).replace("torch.", ""), linear)
+        self._check(self._lib.meao_render_batch(self._ctx, depth.data_ptr(), kind, frames, out.data_ptr(), self._stream(stream)))
+        return out
+
+    def reserve_batch(self, frames: int) -> None:
+        """Allocates the batch intermediates for >= frames frames now (render_batch would on first use)."""
+        self._update(False)
+        self._check(self._lib.meao_reserve_batch(self._ctx, int(frames)))
+
+    def batch_buffer(self, frame: int, debug_id: int) -> np.ndarray:
+        """Buffer <id> (1-16, 18-21) of frame <frame> of the last render_batch, like debug_buffer."""
+        d = self.buffer_desc(debug_id)
+        dt = {1: np.uint8, 2: np.float16, 4: np.float32}[d.elem_bytes]
+        shape = (d.slices, d.height, d.width) if d.slices > 1 else (d.height, d.width)
+        a = np.empty(shape, dt)
+        self._check(self._lib.meao_get_batch_buffer(self._ctx, int(frame), debug_id, a.ctypes.data, a.nbytes))
+        return a
+
     def render_host(self, depth: np.ndarray, out: np.ndarray | None = None, *, linear: bool = False) -> np.ndarray:
         """Host [H, W] depth (float32 / uint16 D16 codes / uint32 D24S8 words) in, host uint8 [H, W] out
         (H2D + the kernels + D2H + sync)."""

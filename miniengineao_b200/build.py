@@ -13,8 +13,8 @@ import sys
 HERE = os.path.dirname(os.path.abspath(__file__))
 CSRC = os.path.join(HERE, "csrc")
 LIB = os.path.join(HERE, "libmeao.so")
-SOURCES = ["meao_api.cu", "prepare_depth.cu", "render_ao.cu", "blur_upsample.cu", "selftest.cu", "halo.cu", "band_exchange.cu", "composite.cu", "debug_view.cu"]
-HEADERS = ["common.cuh", "kernels.h", "blur_upsample_kernel.inc", os.path.join("..", "..", "include", "meao.h")]
+SOURCES = ["meao_api.cu", "prepare_depth.cu", "prepare_depth_batch.cu", "render_ao.cu", "render_ao_batch.cu", "blur_upsample.cu", "blur_upsample_batch.cu", "selftest.cu", "halo.cu", "band_exchange.cu", "composite.cu", "debug_view.cu"]
+HEADERS = ["common.cuh", "kernels.h", "blur_upsample_kernel.inc", "prepare_depth_kernel.inc", "render_ao_kernel.inc", os.path.join("..", "..", "include", "meao.h")]
 
 NVCC_FLAGS = [
     "-gencode", "arch=compute_100a,code=sm_100a",

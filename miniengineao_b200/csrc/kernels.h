@@ -132,6 +132,19 @@ cudaError_t launch_blur_upsample(const CUtensorMap &lo_depth_map, const CUtensor
 constexpr int kUpsDepthBoxW = 40, kUpsDepthBoxH = 22; // TMA boxes of the upsample kernel
 constexpr int kUpsAoBoxW = 64, kUpsAoBoxH = 22;
 
+// ---- batched frames (meao_render_batch): the three stages over `frames` frames in one launch each -------------------
+// Every intermediate of frame f lives at base + f * slot_bytes (one frame slot of the batch arena holds all of them, with the
+// single-frame pitches).  The TMA'd buffers get 3-D maps (w, h, capacity) with strides (pitch, slot_bytes).  The argument
+// blocks wrap the single-frame ones, whose pointers then address frame 0.
+struct PrepareBatchArgs { PrepareArgs base; long long in_frame_bytes; long long slot_bytes; };   // base.vec_ok: holds for EVERY frame
+cudaError_t launch_prepare_depth_batch(const PrepareBatchArgs &a, int frames, cudaStream_t s);
+struct RenderBatchArgs { RenderArgs base; long long slot_bytes; };                               // low and occ advance by slot_bytes
+cudaError_t launch_render_ao_batch(const CUtensorMap &low_map3, bool use_tma, const RenderBatchArgs &a, int frames, cudaStream_t s);
+// lo_depth / lo_ao / lo_ao2 / hi_depth / hi_ao advance by slot_bytes, out by out_frame_bytes (base.out_vec_ok: for every frame)
+struct UpsampleBatchArgs { UpsamplePreminArgs pa; long long slot_bytes; long long out_frame_bytes; int frames; int tiles_per_frame; };
+cudaError_t launch_blur_upsample_batch(const CUtensorMap &lo_depth_map3, const CUtensorMap &lo_ao_map3, const CUtensorMap *lo_ao2_map3,
+                                       bool use_tma, const UpsampleBatchArgs &a, cudaStream_t s);
+
 // ---- debug: synthesise a TiledDepth<k> view (reference layout [16][sh][sw], f16 bits) ----------
 cudaError_t launch_synth_tiled(const float *low, int lw, int lh, int lpitch, int sw, int sh, float pad,
                                __half *out, cudaStream_t s);
@@ -189,8 +202,11 @@ cudaError_t launch_band_exchange(const XchgArgs &a, cudaStream_t s);
 #ifndef MEAO_EMULATE
 template <class K> inline cudaError_t preload_kernel(K kernel) { cudaFuncAttributes at; return cudaFuncGetAttributes(&at, (const void *)kernel); }
 cudaError_t preload_prepare_depth();
+cudaError_t preload_prepare_depth_batch();
 cudaError_t preload_render_ao();
+cudaError_t preload_render_ao_batch();
 cudaError_t preload_blur_upsample();
+cudaError_t preload_blur_upsample_batch();
 cudaError_t preload_band_kernels();
 cudaError_t preload_aux_kernels();      // composite, debug views, self test
 #endif

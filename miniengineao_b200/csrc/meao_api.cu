@@ -57,6 +57,30 @@ struct Plan {
     float zb[4];
 };
 
+// Batch arena (meao_render_batch): `capacity` frame slots of every intermediate, apart from the single-frame arena so that a
+// batch never disturbs meao_get_buffer / debug views / stage calls / the band flags.  Frame f of a buffer is at ptr + f * slot_bytes.
+struct BatchArena {
+    void *base = nullptr;
+    size_t bytes = 0, slot_bytes = 0;
+    int capacity = 0;
+    int last_frames = 0;                    // frames of the last batch (meao_get_batch_buffer)
+    int last_kind = MEAO_DEPTH_RAW_F32;
+    uint32_t *tile_ctr = nullptr;           // its own persistent-loop counters: a batch and a single frame never share a word
+    __half *lin = nullptr;
+    float *low[5] = {nullptr};
+    uint8_t *occ[5] = {nullptr}, *comb[4] = {nullptr}, *hq[5] = {nullptr};
+    bool tma_ok = false;
+    // 3-D maps (w, h, capacity), strides (pitch, slot_bytes); same boxes as the single-frame maps
+    CUtensorMap map_low_ren[kRenderTileVariants][5], map_low_wide[kRenderTileVariants][5];
+    CUtensorMap map_low_ups[5], map_ao_ups[5], map_hq_ups[5], map_occ1_ups;
+};
+
+// what the recorders need to know about a batched launch (nullptr: the single-frame path, today's launches)
+struct BatchRun {
+    int frames;
+    long long in_frame_bytes;               // depth stride between frames (W * H * element size)
+};
+
 }  // namespace
 
 struct MeaoCtx {
@@ -122,6 +146,7 @@ struct MeaoCtx {
     Range own_low[5];                       // rows of LowDepth<k> this band produces
 
     int64_t launches = 0;
+    BatchArena batch;
 
     // CUDA graph cache: one instantiated graph per (depth, out, kind), LRU; when it is full the least recently used
     // executable graph is RE-TARGETED in place with cudaGraphExecUpdate (same topology, new pointers: no device
@@ -253,9 +278,16 @@ void disconnect_peers(MeaoCtx *c)
     }
 }
 
+void free_batch(MeaoCtx *c)
+{
+    if (c->batch.base) cudaFree(c->batch.base);
+    c->batch = BatchArena{};
+}
+
 void free_buffers(MeaoCtx *c)
 {
     drop_graph(c);
+    free_batch(c);
     disconnect_peers(c);
     c->band_flags = nullptr;
     if (c->arena) cudaFree(c->arena);
@@ -271,6 +303,18 @@ int make_map(MeaoCtx *c, CUtensorMap *m, CUtensorMapDataType dt, int elem, void 
     cuuint32_t box[2] = {(cuuint32_t)bw, (cuuint32_t)bh};
     cuuint32_t estr[2] = {1, 1};
     CUresult r = c->encode(m, dt, 2, base, dims, strides, box, estr, CU_TENSOR_MAP_INTERLEAVE_NONE,
+                           CU_TENSOR_MAP_SWIZZLE_NONE, CU_TENSOR_MAP_L2_PROMOTION_L2_128B, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
+    return r == CUDA_SUCCESS ? 0 : -1;
+}
+
+int make_map3(MeaoCtx *c, CUtensorMap *m, CUtensorMapDataType dt, int elem, void *base, int w, int h, int pitch_elems, int frames,
+              size_t slot_bytes, int bw, int bh)
+{
+    cuuint64_t dims[3] = {(cuuint64_t)w, (cuuint64_t)h, (cuuint64_t)frames};
+    cuuint64_t strides[2] = {(cuuint64_t)pitch_elems * elem, (cuuint64_t)slot_bytes};
+    cuuint32_t box[3] = {(cuuint32_t)bw, (cuuint32_t)bh, 1};
+    cuuint32_t estr[3] = {1, 1, 1};
+    CUresult r = c->encode(m, dt, 3, base, dims, strides, box, estr, CU_TENSOR_MAP_INTERLEAVE_NONE,
                            CU_TENSOR_MAP_SWIZZLE_NONE, CU_TENSOR_MAP_L2_PROMOTION_L2_128B, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
     return r == CUDA_SUCCESS ? 0 : -1;
 }
@@ -419,18 +463,78 @@ int ensure_ready(MeaoCtx *c)
     return 0;
 }
 
+// Grows the batch arena to >= frames slots.  Synchronous (device synchronise, cudaFree, cudaMalloc): callers keep it out of
+// timed regions with meao_reserve_batch.  The captured batch graphs point into the old arena and are dropped with it.
+int reserve_batch(MeaoCtx *c, int frames)
+{
+    BatchArena &b = c->batch;
+    if (frames <= b.capacity) return 0;
+    CUDA_TRY(c, cudaDeviceSynchronize());
+    for (auto it = c->graphs.begin(); it != c->graphs.end();) {
+        if (it->first.kind >= 400) { cudaGraphExecDestroy(it->second.exec); it = c->graphs.erase(it); } else ++it;
+    }
+    free_batch(c);
+    size_t off = 0;
+    auto take = [&](size_t bytes) { size_t o = off; off += (bytes + 255) / 256 * 256; return o; };
+    const size_t o_lin = take((size_t)c->lin_pitch * c->lh[0] * sizeof(__half));
+    size_t o_low[5], o_occ[5], o_comb[4], o_hq[5];
+    for (int k = 1; k <= 4; k++) {
+        o_low[k] = take((size_t)c->low_pitch[k] * c->lh[k] * sizeof(float));
+        o_occ[k] = take((size_t)c->occ_pitch[k] * c->lh[k]);
+        if (k <= 3) o_comb[k] = take((size_t)c->occ_pitch[k] * c->lh[k]);
+        o_hq[k] = take((size_t)c->occ_pitch[k] * c->lh[k]);
+    }
+    const size_t slot = off;                        // a multiple of 256 bytes
+    const size_t head = 256;                        // persistent-loop tile counters
+    const size_t total = head + slot * (size_t)frames;
+    cudaError_t e = cudaMalloc(&b.base, total);
+    if (e != cudaSuccess) {
+        b.base = nullptr; cudaGetLastError();
+        return fail(c, e == cudaErrorMemoryAllocation ? MEAO_ERR_NOMEM : MEAO_ERR_CUDA, "batch arena cudaMalloc(%zu) failed: %s", total, cudaGetErrorString(e));
+    }
+    CUDA_TRY(c, cudaMemset(b.base, 0, head));
+    b.bytes = total; b.slot_bytes = slot; b.capacity = frames;
+    char *p = (char *)b.base;
+    b.tile_ctr = (uint32_t *)p;
+    p += head;
+    b.lin = (__half *)(p + o_lin);
+    for (int k = 1; k <= 4; k++) {
+        b.low[k] = (float *)(p + o_low[k]);
+        b.occ[k] = (uint8_t *)(p + o_occ[k]);
+        if (k <= 3) b.comb[k] = (uint8_t *)(p + o_comb[k]);
+        b.hq[k] = (uint8_t *)(p + o_hq[k]);
+    }
+    b.tma_ok = false;
+    if (c->encode) {
+        bool ok = true;
+        for (int k = 1; k <= 4 && ok; k++) {
+            for (int t = 0; t < kRenderTileVariants; t++) {
+                ok &= make_map3(c, &b.map_low_ren[t][k], CU_TENSOR_MAP_DATA_TYPE_FLOAT32, 4, b.low[k], c->lw[k], c->lh[k], c->low_pitch[k], frames, slot, kRenderBoxW, render_box_h(kRenderTileHs[t], false)) == 0;
+                ok &= make_map3(c, &b.map_low_wide[t][k], CU_TENSOR_MAP_DATA_TYPE_FLOAT32, 4, b.low[k], c->lw[k], c->lh[k], c->low_pitch[k], frames, slot, kRenderWideBoxW, render_box_h(kRenderTileHs[t], true)) == 0;
+            }
+            ok &= make_map3(c, &b.map_low_ups[k], CU_TENSOR_MAP_DATA_TYPE_FLOAT32, 4, b.low[k], c->lw[k], c->lh[k], c->low_pitch[k], frames, slot, kUpsDepthBoxW, kUpsDepthBoxH) == 0;
+            uint8_t *ao = (k == 4) ? b.occ[4] : b.comb[k];
+            ok &= make_map3(c, &b.map_ao_ups[k], CU_TENSOR_MAP_DATA_TYPE_UINT8, 1, ao, c->lw[k], c->lh[k], c->occ_pitch[k], frames, slot, kUpsAoBoxW, kUpsAoBoxH) == 0;
+            ok &= make_map3(c, &b.map_hq_ups[k], CU_TENSOR_MAP_DATA_TYPE_UINT8, 1, b.hq[k], c->lw[k], c->lh[k], c->occ_pitch[k], frames, slot, kUpsAoBoxW, kUpsAoBoxH) == 0;
+        }
+        ok &= make_map3(c, &b.map_occ1_ups, CU_TENSOR_MAP_DATA_TYPE_UINT8, 1, b.occ[1], c->lw[1], c->lh[1], c->occ_pitch[1], frames, slot, kUpsAoBoxW, kUpsAoBoxH) == 0;
+        b.tma_ok = ok;
+    }
+    return 0;
+}
+
 struct NvtxRange { explicit NvtxRange(const char *n) { nvtxRangePushA(n); } ~NvtxRange() { nvtxRangePop(); } };
 
 // Tile-height variant (index into kRenderTileHs = {32, 16, 8}) of a render launch.  The big levels keep the 64 x 32 tile
 // (least apron overhead: throughput); a level whose grid would not even put one CTA on every SM is latency-bound -- one
 // CTA's serial time IS the kernel time -- so it takes the tallest tile that still gives >= 148 CTAs, else 64 x 8.
 // (Measured at 4K: level 2, 255 CTAs of 64 x 32, is FASTER with the big tile -- 14.0 vs 15.7 us -- levels 3 / 4 gain ~0.5 us.)
-int render_tile_variant(const MeaoCtx *c, int k, int rows)
+int render_tile_variant(const MeaoCtx *c, int k, int rows, int frames = 1)
 {
     const char *force = getenv("MEAO_REN_TILE");               // tuning aid: 0 / 1 / 2 forces a variant for every level
     if (force && force[0] >= '0' && force[0] < '0' + kRenderTileVariants) return force[0] - '0';
     for (int t = 0; t < kRenderTileVariants; t++) {
-        const int ctas = ((c->lw[k] + 63) / 64) * ((rows + kRenderTileHs[t] - 1) / kRenderTileHs[t]);
+        const long long ctas = (long long)((c->lw[k] + 63) / 64) * ((rows + kRenderTileHs[t] - 1) / kRenderTileHs[t]) * frames;   // a batch: all its frames
         if (ctas >= 148) return t;
     }
     return kRenderTileVariants - 1;
@@ -439,7 +543,7 @@ int render_tile_variant(const MeaoCtx *c, int k, int rows)
 // ---- the three recorders ---------------------------------------------------------------------
 
 // PushDownsampleCommands, AO.cs:604-658
-int record_downsample(MeaoCtx *c, const void *depth, int kind, cudaStream_t s)
+int record_downsample(MeaoCtx *c, const void *depth, int kind, cudaStream_t s, const BatchRun *batch = nullptr)
 {
     if (kind < MEAO_DEPTH_RAW_F32 || kind > MEAO_DEPTH_RAW_D24S8) return fail(c, MEAO_ERR_INVALID, "bad depth kind %d", kind);
     NvtxRange nv("meao::prepare_depth");
@@ -455,6 +559,16 @@ int record_downsample(MeaoCtx *c, const void *depth, int kind, cudaStream_t s)
     a.raw = (kind != MEAO_DEPTH_LINEAR_F32);
     a.reversed_z = c->camera.reversed_z;
     a.vec_ok = (((uintptr_t)depth & 15) == 0) && (c->W % (a.in_format == 1 ? 8 : 4) == 0);
+    if (batch) {
+        const BatchArena &b = c->batch;
+        a.lin = b.lin;
+        for (int k = 1; k <= 4; k++) a.low[k - 1] = b.low[k];
+        a.vec_ok = a.vec_ok && (batch->in_frame_bytes % 16 == 0);     // every frame's base stays 16-byte aligned
+        c->batch.last_kind = kind;
+        CUDA_TRY(c, launch_prepare_depth_batch(PrepareBatchArgs{a, batch->in_frame_bytes, (long long)b.slot_bytes}, batch->frames, s));
+        c->launches++;
+        return 0;
+    }
     c->last_kind = kind;
     CUDA_TRY(c, launch_prepare_depth(a, s));
     c->launches++;
@@ -463,7 +577,7 @@ int record_downsample(MeaoCtx *c, const void *depth, int kind, cudaStream_t s)
 
 // PushRenderCommands, AO.cs:660-748.  wide = false: the call AmbientOcclusion.cs makes (tiled source, kernel main_interleaved);
 // wide = true: the same recorder for the non-tiled source LowDepth<k> (kernel main) -> HighQuality<k>.
-int record_render(MeaoCtx *c, int k, int kind, cudaStream_t s, bool wide = false)
+int record_render(MeaoCtx *c, int k, int kind, cudaStream_t s, bool wide = false, const BatchRun *batch = nullptr)
 {
     static const int idx_checker[7] = {1, 3, 4, 8, 11, 6, 10};                       // Render.compute:162-168 table slots, call order
     static const int idx_exh[12] = {0, 1, 2, 3, 4, 8, 11, 5, 6, 7, 9, 10};           // Render.compute:148-159
@@ -487,8 +601,15 @@ int record_render(MeaoCtx *c, int k, int kind, cudaStream_t s, bool wide = false
     a.row0 = c->need_c[k].lo; a.row1 = c->need_c[k].hi;
     a.wide = wide ? 1 : 0;
     a.exhaustive = exh ? 1 : 0;
-    const int tv = render_tile_variant(c, k, a.row1 - (a.row0 & ~3));
+    const int tv = render_tile_variant(c, k, a.row1 - (a.row0 & ~3), batch ? batch->frames : 1);
     a.tile_h = kRenderTileHs[tv];
+    if (batch) {
+        const BatchArena &b = c->batch;
+        a.low = b.low[k]; a.occ = wide ? b.hq[k] : b.occ[k];
+        CUDA_TRY(c, launch_render_ao_batch(wide ? b.map_low_wide[tv][k] : b.map_low_ren[tv][k], b.tma_ok, RenderBatchArgs{a, (long long)b.slot_bytes}, batch->frames, s));
+        c->launches++;
+        return 0;
+    }
     CUDA_TRY(c, launch_render_ao(wide ? c->map_low_wide[tv][k] : c->map_low_ren[tv][k], c->tma_ok, a, s));
     c->launches++;
     return 0;
@@ -496,7 +617,7 @@ int record_render(MeaoCtx *c, int k, int kind, cudaStream_t s, bool wide = false
 inline bool hq_level(const MeaoCtx *c, int k) { return ((c->variants.high_quality_mask >> (k - 1)) & 1) != 0; }
 
 // PushUpsampleCommands with the wiring of AO.cs:528-531
-int record_upsample(MeaoCtx *c, int lo, void *ao_out, cudaStream_t s)
+int record_upsample(MeaoCtx *c, int lo, void *ao_out, cudaStream_t s, const BatchRun *batch = nullptr)
 {
     const int hi = lo - 1;
     NvtxRange nv("meao::blur_upsample");
@@ -509,7 +630,7 @@ int record_upsample(MeaoCtx *c, int lo, void *ao_out, cudaStream_t s)
     if (hi == 0) {
         if (ao_out) { a.out = (uint8_t *)ao_out; a.out_pitch = c->W; a.out_row_origin = c->band0; }
         else { a.out = c->result; a.out_pitch = c->result_pitch; a.out_row_origin = 0; }
-        c->last_out = ao_out;
+        if (!batch) c->last_out = ao_out;
     } else { a.out = c->comb[hi]; a.out_pitch = c->occ_pitch[hi]; a.out_row_origin = 0; }
     a.out_vec_ok = (((uintptr_t)a.out & 7) == 0) && (a.out_pitch % 8 == 0);
     a.hiw = c->lw[hi]; a.hih = c->lh[hi];
@@ -529,6 +650,22 @@ int record_upsample(MeaoCtx *c, int lo, void *ao_out, cudaStream_t s)
     a.row0 = c->need_c[hi].lo; a.row1 = c->need_c[hi].hi;
     a.tile_ctr = c->tile_ctr + 2 * (lo - 1);
     const uint8_t *lo_ao2 = hq_level(c, lo) ? c->hq[lo] : nullptr;                   // kernels main_premin / main_premin_blendout
+    if (batch) {
+        const BatchArena &b = c->batch;
+        a.lo_depth = b.low[lo];
+        a.lo_ao = single ? b.occ[1] : (lo == 4) ? b.occ[4] : b.comb[lo];
+        if (hi == 0) a.hi_depth = b.lin;
+        else { a.hi_depth = b.low[hi]; a.hi_ao = b.occ[hi]; }
+        long long out_frame_bytes = (long long)b.slot_bytes;
+        if (hi == 0) { a.out = (uint8_t *)ao_out; a.out_pitch = c->W; a.out_row_origin = 0; out_frame_bytes = (long long)c->W * c->H; }
+        else a.out = b.comb[hi];
+        a.out_vec_ok = (((uintptr_t)a.out & 7) == 0) && (a.out_pitch % 8 == 0) && (out_frame_bytes % 8 == 0);
+        a.tile_ctr = b.tile_ctr + 2 * (lo - 1);
+        UpsampleBatchArgs ba{UpsamplePreminArgs{a, hq_level(c, lo) ? b.hq[lo] : nullptr, c->occ_pitch[lo]}, (long long)b.slot_bytes, out_frame_bytes, batch->frames, 0};
+        CUDA_TRY(c, launch_blur_upsample_batch(b.map_low_ups[lo], single ? b.map_occ1_ups : b.map_ao_ups[lo], &b.map_hq_ups[lo], b.tma_ok, ba, s));
+        c->launches++;
+        return 0;
+    }
     CUDA_TRY(c, launch_blur_upsample(c->map_low_ups[lo], single ? c->map_occ1_ups : c->map_ao_ups[lo], &c->map_hq_ups[lo], c->tma_ok, a, lo_ao2, c->occ_pitch[lo], s));
     c->launches++;
     return 0;
@@ -545,45 +682,45 @@ struct PdlScope { bool prev; explicit PdlScope(bool on) : prev(g_launch_pdl) { g
 // before this DAG is the neighbour-exchange kernel, which spins on remote flags -- nothing may be scheduled "early" behind it
 // (a grid parked in griddepcontrol.wait holds SM resources that the neighbour band's kernels may need: see DESIGN.md 4).
 int record_frame_dag(MeaoCtx *c, const void *depth, int kind, void *ao_out, cudaStream_t s, bool do_prepare = true, int pdl = 0,
-                     bool after_exchange = false)
+                     bool after_exchange = false, const BatchRun *batch = nullptr)
 {
     int rc;
     if (c->variants.single_scale) {     // BASELINE.json configs[0]: Downsample1 -> Render level 1 -> final-style Upsample on Occlusion1
-        if (do_prepare && (rc = record_downsample(c, depth, kind, s))) return rc;
-        { PdlScope p(pdl >= 1 && !after_exchange); if ((rc = record_render(c, 1, kind, s))) return rc; }
-        { PdlScope p(pdl >= 1); if ((rc = record_upsample(c, 1, ao_out, s))) return rc; }
+        if (do_prepare && (rc = record_downsample(c, depth, kind, s, batch))) return rc;
+        { PdlScope p(pdl >= 1 && !after_exchange); if ((rc = record_render(c, 1, kind, s, false, batch))) return rc; }
+        { PdlScope p(pdl >= 1); if ((rc = record_upsample(c, 1, ao_out, s, batch))) return rc; }
         return 0;
     }
     cudaStream_t b1 = c->branch[0], b2 = c->branch[1], b3 = c->branch[2];
-    if (do_prepare && (rc = record_downsample(c, depth, kind, s))) return rc;
+    if (do_prepare && (rc = record_downsample(c, depth, kind, s, batch))) return rc;
     CUDA_TRY(c, cudaEventRecord(c->ev[0], s));
     CUDA_TRY(c, cudaStreamWaitEvent(b1, c->ev[0], 0));
     CUDA_TRY(c, cudaStreamWaitEvent(b2, c->ev[0], 0));
     CUDA_TRY(c, cudaStreamWaitEvent(b3, c->ev[0], 0));
     // the optional high-quality render of a level (kernel "main") rides on the branch of that level's interleaved render
-    { PdlScope p(pdl >= 1 && !after_exchange); if ((rc = record_render(c, 1, kind, s))) return rc; }
-    { PdlScope p(pdl >= 1); if (hq_level(c, 1) && (rc = record_render(c, 1, kind, s, true))) return rc; }
-    if ((rc = record_render(c, 2, kind, b1))) return rc;
-    { PdlScope p(pdl >= 1); if (hq_level(c, 2) && (rc = record_render(c, 2, kind, b1, true))) return rc; }
+    { PdlScope p(pdl >= 1 && !after_exchange); if ((rc = record_render(c, 1, kind, s, false, batch))) return rc; }
+    { PdlScope p(pdl >= 1); if (hq_level(c, 1) && (rc = record_render(c, 1, kind, s, true, batch))) return rc; }
+    if ((rc = record_render(c, 2, kind, b1, false, batch))) return rc;
+    { PdlScope p(pdl >= 1); if (hq_level(c, 2) && (rc = record_render(c, 2, kind, b1, true, batch))) return rc; }
     CUDA_TRY(c, cudaEventRecord(c->ev[1], b1));
-    if ((rc = record_render(c, 3, kind, b2))) return rc;
-    { PdlScope p(pdl >= 1); if (hq_level(c, 3) && (rc = record_render(c, 3, kind, b2, true))) return rc; }
+    if ((rc = record_render(c, 3, kind, b2, false, batch))) return rc;
+    { PdlScope p(pdl >= 1); if (hq_level(c, 3) && (rc = record_render(c, 3, kind, b2, true, batch))) return rc; }
     CUDA_TRY(c, cudaEventRecord(c->ev[2], b2));
-    if ((rc = record_render(c, 4, kind, b3))) return rc;
-    { PdlScope p(pdl >= 1); if (hq_level(c, 4) && (rc = record_render(c, 4, kind, b3, true))) return rc; }
+    if ((rc = record_render(c, 4, kind, b3, false, batch))) return rc;
+    { PdlScope p(pdl >= 1); if (hq_level(c, 4) && (rc = record_render(c, 4, kind, b3, true, batch))) return rc; }
     CUDA_TRY(c, cudaStreamWaitEvent(b3, c->ev[2], 0));
-    { PdlScope p(pdl >= 2); if ((rc = record_upsample(c, 4, nullptr, b3))) return rc; }
+    { PdlScope p(pdl >= 2); if ((rc = record_upsample(c, 4, nullptr, b3, batch))) return rc; }
     CUDA_TRY(c, cudaStreamWaitEvent(b3, c->ev[1], 0));
-    { PdlScope p(pdl >= 2); if ((rc = record_upsample(c, 3, nullptr, b3))) return rc; }
+    { PdlScope p(pdl >= 2); if ((rc = record_upsample(c, 3, nullptr, b3, batch))) return rc; }
     CUDA_TRY(c, cudaEventRecord(c->ev[3], b3));
     CUDA_TRY(c, cudaStreamWaitEvent(s, c->ev[3], 0));
-    { PdlScope p(pdl >= 2); if ((rc = record_upsample(c, 2, nullptr, s))) return rc; }
-    { PdlScope p(pdl >= 1); if ((rc = record_upsample(c, 1, ao_out, s))) return rc; }
+    { PdlScope p(pdl >= 2); if ((rc = record_upsample(c, 2, nullptr, s, batch))) return rc; }
+    { PdlScope p(pdl >= 1); if ((rc = record_upsample(c, 1, ao_out, s, batch))) return rc; }
     return 0;
 }
 
 // record order of RebuildCommandBuffers, AO.cs:511-531
-int record_frame(MeaoCtx *c, const void *depth, int kind, void *ao_out, cudaStream_t s, bool profile)
+int record_frame(MeaoCtx *c, const void *depth, int kind, void *ao_out, cudaStream_t s, bool profile, const BatchRun *batch = nullptr)
 {
     static const char *ren_names[5] = {"", "render_ao L1", "render_ao L2", "render_ao L3", "render_ao L4"};
     static const char *hq_names[5] = {"", "render_ao_wide L1", "render_ao_wide L2", "render_ao_wide L3", "render_ao_wide L4"};
@@ -594,13 +731,13 @@ int record_frame(MeaoCtx *c, const void *depth, int kind, void *ao_out, cudaStre
     const int reps = profile ? c->profile_repeats : 1;         // every kernel is idempotent (out of place), so repeating it is harmless
     int rc = 0;
     mark();
-    for (int r = 0; r < reps && !rc; r++) rc = record_downsample(c, depth, kind, s);
+    for (int r = 0; r < reps && !rc; r++) rc = record_downsample(c, depth, kind, s, batch);
     if (rc) return rc;
     names.push_back("prepare_depth"); mark();
     const int kmax = c->variants.single_scale ? 1 : 4;       // single-scale: Render level 1 + the final-style Upsample only
-    for (int k = 1; k <= kmax; k++) { for (int r = 0; r < reps && !rc; r++) rc = record_render(c, k, kind, s); if (rc) return rc; names.push_back(ren_names[k]); mark(); }
-    for (int k = 1; k <= kmax; k++) if (hq_level(c, k)) { for (int r = 0; r < reps && !rc; r++) rc = record_render(c, k, kind, s, true); if (rc) return rc; names.push_back(hq_names[k]); mark(); }
-    for (int lo = kmax; lo >= 1; lo--) { for (int r = 0; r < reps && !rc; r++) rc = record_upsample(c, lo, lo == 1 ? ao_out : nullptr, s); if (rc) return rc; names.push_back(ups_names[lo]); mark(); }
+    for (int k = 1; k <= kmax; k++) { for (int r = 0; r < reps && !rc; r++) rc = record_render(c, k, kind, s, false, batch); if (rc) return rc; names.push_back(ren_names[k]); mark(); }
+    for (int k = 1; k <= kmax; k++) if (hq_level(c, k)) { for (int r = 0; r < reps && !rc; r++) rc = record_render(c, k, kind, s, true, batch); if (rc) return rc; names.push_back(hq_names[k]); mark(); }
+    for (int lo = kmax; lo >= 1; lo--) { for (int r = 0; r < reps && !rc; r++) rc = record_upsample(c, lo, lo == 1 ? ao_out : nullptr, s, batch); if (rc) return rc; names.push_back(ups_names[lo]); mark(); }
     if (profile) {
         CUDA_TRY(c, cudaStreamSynchronize(s));
         c->last_profile.clear();
@@ -717,6 +854,9 @@ int meao_create(const MeaoDeviceCfg *cfg, MeaoCtx **out)
             cudaError_t pe = preload_prepare_depth();
             if (pe == cudaSuccess) pe = preload_render_ao();
             if (pe == cudaSuccess) pe = preload_blur_upsample();
+            if (pe == cudaSuccess) pe = preload_blur_upsample_batch();
+            if (pe == cudaSuccess) pe = preload_prepare_depth_batch();
+            if (pe == cudaSuccess) pe = preload_render_ao_batch();
             if (pe == cudaSuccess) pe = preload_band_kernels();
             if (pe == cudaSuccess) pe = preload_aux_kernels();
             if (pe != cudaSuccess) { cudaGetLastError(); meao_destroy(c); return fail(nullptr, MEAO_ERR_CUDA, "loading the kernels failed: %s", cudaGetErrorString(pe)); }
@@ -1229,6 +1369,70 @@ int meao_render(MeaoCtx *c, const void *depth, int32_t kind, void *ao_out, void 
     return launch_cached(c, key, s, meao_kernels_per_frame(c), [&](cudaStream_t cs, int pdl) {
         return record_frame_dag(c, depth, kind, ao_out, cs, true, pdl);
     });
+}
+
+int meao_reserve_batch(MeaoCtx *c, int32_t frames)
+{
+    int rc = ensure_ready(c); if (rc) return rc;
+    if (frames < 1 || frames > 65535) return fail(c, MEAO_ERR_INVALID, "frames %d not in 1..65535", frames);
+    return reserve_batch(c, frames);
+}
+
+int meao_render_batch(MeaoCtx *c, const void *depth, int32_t kind, int32_t frames, void *ao_out, void *stream)
+{
+    int rc = ensure_ready(c); if (rc) return rc;
+    if (!depth || !ao_out) return fail(c, MEAO_ERR_INVALID, "depth / ao_out is NULL");
+    if (kind < MEAO_DEPTH_RAW_F32 || kind > MEAO_DEPTH_RAW_D24S8) return fail(c, MEAO_ERR_INVALID, "bad depth kind %d", kind);
+    if (frames < 1 || frames > 65535) return fail(c, MEAO_ERR_INVALID, "frames %d not in 1..65535", frames);
+    if (c->band0 != 0 || c->band1 != c->H) return fail(c, MEAO_ERR_UNSUPPORTED, "batched frames need a whole-frame context (no row band)");
+    if ((rc = reserve_batch(c, frames))) return rc;
+    cudaStream_t s = (cudaStream_t)stream;
+    const size_t esz = (kind == MEAO_DEPTH_RAW_D16_UNORM) ? 2 : 4;
+    const BatchRun run{frames, (long long)c->W * c->H * (long long)esz};
+    c->batch.last_frames = frames;
+    if (c->flags & MEAO_FLAG_NO_GRAPH) return record_frame(c, depth, kind, ao_out, s, false, &run);
+    // one graph replay for the whole batch: the DAG of record_frame_dag, every node covering all frames
+    NvtxRange nv("meao::batch");
+    const MeaoCtx::GraphKey key{{depth, ao_out, (const void *)(uintptr_t)frames, c->batch.base}, 400 + kind};
+    return launch_cached(c, key, s, meao_kernels_per_frame(c), [&](cudaStream_t cs, int pdl) {
+        return record_frame_dag(c, depth, kind, ao_out, cs, true, pdl, false, &run);
+    });
+}
+
+int meao_get_batch_buffer(MeaoCtx *c, int32_t frame, int32_t id, void *host_out, size_t host_bytes)
+{
+    int rc = ensure_ready(c); if (rc) return rc;
+    int lvl, slices, elem;
+    if (!host_out || id == MEAO_BUF_AMBIENT_OCCLUSION || buffer_info(c, id, &lvl, &slices, &elem))
+        return fail(c, MEAO_ERR_INVALID, "bad batch buffer id %d (the AO of a batch is in the caller's buffer)", id);
+    const BatchArena &b = c->batch;
+    if (frame < 0 || frame >= b.last_frames) return fail(c, MEAO_ERR_INVALID, "frame %d not in the last batch (%d frames)", frame, b.last_frames);
+    const size_t need = (size_t)c->lw[lvl] * c->lh[lvl] * slices * elem;
+    if (host_bytes < need) return fail(c, MEAO_ERR_INVALID, "buffer %d needs %zu bytes, got %zu", id, need, host_bytes);
+    CUDA_TRY(c, cudaDeviceSynchronize());     // debug path: batches may be in flight on any caller stream
+    const size_t fo = (size_t)frame * b.slot_bytes;
+    if (slices == 16) {
+        const int k = id - 5;
+        __half *tmp = nullptr;
+        CUDA_TRY(c, cudaMalloc(&tmp, need));
+        const float pad = host_f16_round((b.last_kind != MEAO_DEPTH_LINEAR_F32) ? c->plan.pad[k] : 0.0f);
+        cudaError_t e = launch_synth_tiled((const float *)((const char *)b.low[k] + fo), c->lw[k], c->lh[k], c->low_pitch[k], c->lw[k + 2], c->lh[k + 2], pad, tmp, c->stream);
+        if (e == cudaSuccess) e = cudaMemcpyAsync(host_out, tmp, need, cudaMemcpyDeviceToHost, c->stream);
+        if (e == cudaSuccess) e = cudaStreamSynchronize(c->stream);
+        cudaFree(tmp);
+        if (e != cudaSuccess) return fail(c, MEAO_ERR_CUDA, "tiled view: %s", cudaGetErrorString(e));
+        return MEAO_OK;
+    }
+    const void *p; size_t pitch;
+    if (id == 1) { p = b.lin; pitch = (size_t)c->lin_pitch * 2; }
+    else if (id >= 2 && id <= 5) { p = b.low[id - 1]; pitch = (size_t)c->low_pitch[id - 1] * 4; }
+    else if (id >= 10 && id <= 13) { p = b.occ[id - 9]; pitch = c->occ_pitch[id - 9]; }
+    else if (id >= 14 && id <= 16) { p = b.comb[id - 13]; pitch = c->occ_pitch[id - 13]; }
+    else { p = b.hq[id - 17]; pitch = c->occ_pitch[id - 17]; }
+    const size_t wb = (size_t)c->lw[lvl] * elem;
+    CUDA_TRY(c, cudaMemcpy2DAsync(host_out, wb, (const char *)p + fo, pitch, wb, c->lh[lvl], cudaMemcpyDeviceToHost, c->stream));
+    CUDA_TRY(c, cudaStreamSynchronize(c->stream));
+    return MEAO_OK;
 }
 
 int meao_render_host_async(MeaoCtx *c, const void *depth_host, int32_t kind, uint8_t *ao_host, int32_t slot)

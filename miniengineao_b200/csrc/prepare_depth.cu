@@ -112,80 +112,15 @@ __device__ __forceinline__ void load8(const void *base, size_t elem_index, bool 
     }
 }
 
-template <bool RAW, bool REVERSED, int IN>
-__global__ void __launch_bounds__(kPrepThreads) prepare_depth_kernel(const PrepareArgs a)
-{
-#ifdef MEAO_DEVICE_OK
-    const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
-    const int x = blockIdx.x * kPrepTileW + lane * 8;
-    const int ybase = a.row0 + blockIdx.y * kPrepTileH;
-    pdl_wait();                     // (first node of the frame's graph: a no-op today; keeps the rule "wait before the first global access")
-    pdl_launch_dependents();
-    if (x >= a.W) return;
-    const bool full = a.vec_ok && (x + 8 <= a.W);
-
-    float v[2][8];
-    bool rowok[2];
-#pragma unroll
-    for (int p = 0; p < 2; p++) {
-        const int y = ybase + warp + 8 * p;
-        rowok[p] = y < a.row1;
-        if (rowok[p]) load8<IN>(a.depth, (size_t)(y - a.depth_row0) * a.W + x, full, a.W - x, v[p]);
-    }
-
-#pragma unroll
-    for (int p = 0; p < 2; p++) {
-        if (!rowok[p]) continue;
-        const int y = ybase + warp + 8 * p;
-        float d[8];
-#if MEAO_PACKED_RCP
-        linearize8<RAW, REVERSED>(v[p], a.zbx, a.zby, d);
-#else
-#pragma unroll
-        for (int e = 0; e < 8; e++) d[e] = linearize<RAW, REVERSED>(v[p][e], a.zbx, a.zby);
+// (built a second time with MEAO_PREP_BATCH = 1 by prepare_depth_batch.cu: the batched kernels and their launcher)
+#ifndef MEAO_PREP_BATCH
+#define MEAO_PREP_BATCH 0
 #endif
-
-        __half *lin = a.lin + (size_t)y * a.lin_pitch + x;
-        if (full) {
-            __half2 h0 = __floats2half2_rn(d[0], d[1]), h1 = __floats2half2_rn(d[2], d[3]);
-            __half2 h2 = __floats2half2_rn(d[4], d[5]), h3 = __floats2half2_rn(d[6], d[7]);
-            uint4 pk;
-            pk.x = *reinterpret_cast<uint32_t *>(&h0); pk.y = *reinterpret_cast<uint32_t *>(&h1);
-            pk.z = *reinterpret_cast<uint32_t *>(&h2); pk.w = *reinterpret_cast<uint32_t *>(&h3);
-            *reinterpret_cast<uint4 *>(lin) = pk;                                        // DS1:46
-            if ((y & 1) == 0) {                                                          // DS1:70  DS2x
-                float *l1 = a.low[0] + (size_t)(y >> 1) * a.low_pitch[0] + (x >> 1);
-                *reinterpret_cast<float4 *>(l1) = make_float4(d[0], d[2], d[4], d[6]);
-                if ((y & 3) == 0) {                                                      // DS1:77  DS4x
-                    float *l2 = a.low[1] + (size_t)(y >> 2) * a.low_pitch[1] + (x >> 2);
-                    *reinterpret_cast<float2 *>(l2) = make_float2(d[0], d[4]);
-                    if ((y & 7) == 0) {                                                  // DS2:40  DS8x
-                        a.low[2][(size_t)(y >> 3) * a.low_pitch[2] + (x >> 3)] = d[0];
-                        if ((y & 15) == 0 && (lane & 1) == 0)                            // DS2:48  DS16x
-                            a.low[3][(size_t)(y >> 4) * a.low_pitch[3] + (x >> 4)] = d[0];
-                    }
-                }
-            }
-        } else {
-#pragma unroll
-            for (int e = 0; e < 8; e++) {
-                const int xx = x + e;
-                if (xx >= a.W) break;
-                lin[e] = __float2half_rn(d[e]);
-#pragma unroll
-                for (int k = 1; k <= 4; k++) {
-                    const int m = (1 << k) - 1;
-                    if ((xx & m) == 0 && (y & m) == 0)
-                        a.low[k - 1][(size_t)(y >> k) * a.low_pitch[k - 1] + (xx >> k)] = d[e];
-                }
-            }
-        }
-    }
-#endif
-}
+#include "prepare_depth_kernel.inc"
 
 }  // namespace
 
+#if !MEAO_PREP_BATCH
 cudaError_t launch_prepare_depth(const PrepareArgs &a, cudaStream_t s)
 {
     if (a.row1 <= a.row0) return cudaSuccess;
@@ -216,6 +151,40 @@ cudaError_t preload_prepare_depth()
     t(prepare_depth_kernel<true, true, IN_D24S8>); t(prepare_depth_kernel<true, false, IN_D24S8>);
     return e;
 }
+#endif
+#else   // prepare_depth_batch.cu
+cudaError_t launch_prepare_depth_batch(const PrepareBatchArgs &b, int frames, cudaStream_t s)
+{
+    const PrepareArgs &a = b.base;
+    if (a.row1 <= a.row0 || frames < 1) return cudaSuccess;
+    dim3 grid(ceil_div(a.W, kPrepTileW), ceil_div(a.row1 - a.row0, kPrepTileH), frames);
+    if (!a.raw) {
+        MEAO_LAUNCH((prepare_depth_batch_kernel<false, true, IN_F32>), grid, kPrepThreads, 0, s, b);
+    } else if (a.in_format == IN_D16) {
+        if (a.reversed_z) MEAO_LAUNCH((prepare_depth_batch_kernel<true, true, IN_D16>), grid, kPrepThreads, 0, s, b);
+        else              MEAO_LAUNCH((prepare_depth_batch_kernel<true, false, IN_D16>), grid, kPrepThreads, 0, s, b);
+    } else if (a.in_format == IN_D24S8) {
+        if (a.reversed_z) MEAO_LAUNCH((prepare_depth_batch_kernel<true, true, IN_D24S8>), grid, kPrepThreads, 0, s, b);
+        else              MEAO_LAUNCH((prepare_depth_batch_kernel<true, false, IN_D24S8>), grid, kPrepThreads, 0, s, b);
+    } else {
+        if (a.reversed_z) MEAO_LAUNCH((prepare_depth_batch_kernel<true, true, IN_F32>), grid, kPrepThreads, 0, s, b);
+        else              MEAO_LAUNCH((prepare_depth_batch_kernel<true, false, IN_F32>), grid, kPrepThreads, 0, s, b);
+    }
+    return cudaGetLastError();
+}
+
+#ifndef MEAO_EMULATE
+cudaError_t preload_prepare_depth_batch()
+{
+    cudaError_t e = cudaSuccess;
+    auto t = [&](auto k) { if (e == cudaSuccess) e = preload_kernel(k); };
+    t(prepare_depth_batch_kernel<false, true, IN_F32>);
+    t(prepare_depth_batch_kernel<true, true, IN_F32>); t(prepare_depth_batch_kernel<true, false, IN_F32>);
+    t(prepare_depth_batch_kernel<true, true, IN_D16>); t(prepare_depth_batch_kernel<true, false, IN_D16>);
+    t(prepare_depth_batch_kernel<true, true, IN_D24S8>); t(prepare_depth_batch_kernel<true, false, IN_D24S8>);
+    return e;
+}
+#endif
 #endif
 
 }  // namespace meao

@@ -124,135 +124,13 @@ __device__ __forceinline__ void lshape2(const float *c, float2 inv, float it, fl
     ao = __ffma2_rn(make_float2(w, w), __fmul2_rn(make_float2(0.25f, 0.25f), t), ao);
 }
 
-template <int MODE, bool EXH, int TH>
-__global__ void __launch_bounds__(kThreads, MEAO_REN_MINB)
-render_ao_kernel(const __grid_constant__ CUtensorMap low_map, const RenderArgs a, const int use_tma)
-{
-#ifdef MEAO_DEVICE_OK
-    static_assert(TH % kWarps == 0, "rows must split evenly over the warps");
-    constexpr int kTH = TH;
-    constexpr int kAp = Geo<MODE, TH>::kAp, kSW = Geo<MODE, TH>::kSW, kSH = Geo<MODE, TH>::kSH;
-#ifdef MEAO_EMULATE
-    float *tile = reinterpret_cast<float *>(meao_emu::dynamic_smem());
-#else
-    extern __shared__ __align__(128) float tile[];     // kSW * kSH floats
+// (built a second time with MEAO_REN_BATCH = 1 by render_ao_batch.cu: the batched kernels and their launcher)
+#ifndef MEAO_REN_BATCH
+#define MEAO_REN_BATCH 0
 #endif
-    __shared__ __align__(8) uint64_t bar;
+#include "render_ao_kernel.inc"
 
-    const int tid = threadIdx.x;
-    const int X0 = blockIdx.x * kTW;
-    const int Y0 = (a.row0 & ~3) + blockIdx.y * kTH;
-
-    const bool interior = use_tma && (X0 - kAp >= 0) && (Y0 - kAp >= 0) && (X0 + kTW + kAp <= a.lw) && (Y0 + kTH + kAp <= a.lh);
-
-    pdl_wait();                     // LowDepth<k> comes from the preceding grid(s); nothing above touches global memory
-    pdl_launch_dependents();
-    if (interior) {
-        // ---- TMA: one 96x64 (wide: 80x48) f32 box, completion on an mbarrier ------------------
-        if (tid == 0) {
-            mbar_init(&bar, 1);
-            fence_mbar_init();
-        }
-        __syncthreads();
-        if (tid == 0) {
-            mbar_arrive_expect_tx(&bar, kSW * kSH * (uint32_t)sizeof(float));
-            tma_load_2d(tile, &low_map, X0 - kAp, Y0 - kAp, &bar);
-        }
-        mbar_wait(&bar, 0);
-        if (MODE == 0) {
-            // in-place f16 rounding (what the RHalf atlas store of DS1:71 / DS2:41 does)
-            float4 *t4 = reinterpret_cast<float4 *>(tile);
-            constexpr int kQuads = kSW * kSH / 4;
-#pragma unroll
-            for (int i = 0; i < (kQuads + kThreads - 1) / kThreads; i++) {
-                if (kQuads % kThreads != 0 && tid + i * kThreads >= kQuads) break;
-                float4 q = t4[tid + i * kThreads];
-                q.x = f16_round(q.x); q.y = f16_round(q.y); q.z = f16_round(q.z); q.w = f16_round(q.w);
-                t4[tid + i * kThreads] = q;
-            }
-        }
-    } else if (MODE == 1) {
-        // ---- border tile, kernel `main`: per-texel clamp-to-edge of the Gather (REN:125), f32 as stored ----
-        // (unrolled: the loads of several iterations are in flight together -- one dependent L2 round trip per iteration made the
-        //  border CTAs, i.e. nearly every CTA of the coarse levels, several microseconds slower than the TMA-fed ones)
-#pragma unroll 8
-        for (int idx = tid; idx < kSW * kSH; idx += kThreads) {
-            const int tx = idx % kSW, ty = idx / kSW;
-            const int sx = iclamp(X0 - kAp + tx, 0, a.lw - 1), sy = iclamp(Y0 - kAp + ty, 0, a.lh - 1);
-            tile[idx] = __ldg(a.low + (size_t)sy * a.lpitch + sx);
-        }
-    } else {
-        // ---- border tile: resolve slice-space clamp + atlas padding per texel ------------------
-#pragma unroll 8
-        for (int idx = tid; idx < kSW * kSH; idx += kThreads) {
-            const int tx = idx % kSW, ty = idx / kSW;
-            const int vx = X0 - kAp + tx, vy = Y0 - kAp + ty;
-            const int sx = 4 * iclamp(vx >> 2, 0, a.sw - 1) + (vx & 3);     // clamp addressing of Gather, REN:123
-            const int sy = 4 * iclamp(vy >> 2, 0, a.sh - 1) + (vy & 3);
-            float v = a.pad;
-            if (sx < a.lw && sy < a.lh) v = f16_round(__ldg(a.low + (size_t)sy * a.lpitch + sx));
-            tile[idx] = v;
-        }
-    }
-    __syncthreads();
-
-    // ---- sampling: thread -> pixels (2*lane, 2*lane+1) of rows wy, wy+8, wy+16, wy+24 -------------
-    const int lane = tid & 31, wy = tid >> 5;
-    const int px = 2 * lane;
-    const float rf = a.reject_fadeoff;
-#pragma unroll 1
-    for (int i = 0; i < kTH / kWarps; i++) {
-        const int row = wy + kWarps * i;
-        const int oy = Y0 + row, ox = X0 + px;
-        if (oy < a.row0 || oy >= a.row1 || ox >= a.lw) continue;
-        const float *c = tile + (row + kAp) * kSW + (px + kAp);
-        const float2 ctr = *reinterpret_cast<const float2 *>(c);
-#if MEAO_PACKED_RCP
-        float2 inv;                                                            // REN:140, both pixels under one range test
-        {
-            const float2 nctr = __fmul2_rn(ctr, make_float2(-1.0f, -1.0f));
-            if (in_safe_range_neg(nctr.x) & in_safe_range_neg(nctr.y)) inv = rcp2_fast_neg(nctr);
-            else inv = make_float2(1.0f / ctr.x, 1.0f / ctr.y);
-        }
-#else
-        const float2 inv = make_float2(rcp_ieee(ctr.x), rcp_ieee(ctr.y));      // REN:140
-#endif
-        float2 ao = make_float2(0.0f, 0.0f);                                   // REN:142
-        if (!EXH) {
-            // REN:162-168 -- the 36-sample checker pattern, in call order
-            axial2<MODE, 2>(c, inv, a.inv_thickness[0], a.neg_front[0], a.weight[0], rf, ao);
-            axial2<MODE, 4>(c, inv, a.inv_thickness[1], a.neg_front[1], a.weight[1], rf, ao);
-            diag2<MODE, 1>(c, inv, a.inv_thickness[2], a.neg_front[2], a.weight[2], rf, ao);
-            diag2<MODE, 2>(c, inv, a.inv_thickness[3], a.neg_front[3], a.weight[3], rf, ao);
-            diag2<MODE, 3>(c, inv, a.inv_thickness[4], a.neg_front[4], a.weight[4], rf, ao);
-            lshape2<MODE, 1, 3>(c, inv, a.inv_thickness[5], a.neg_front[5], a.weight[5], rf, ao);
-            lshape2<MODE, 2, 4>(c, inv, a.inv_thickness[6], a.neg_front[6], a.weight[6], rf, ao);
-        } else {
-            // REN:148-159 -- SAMPLE_EXHAUSTIVELY: all 68 cells within radius 5, in call order
-            axial2<MODE, 1>(c, inv, a.inv_thickness[0], a.neg_front[0], a.weight[0], rf, ao);
-            axial2<MODE, 2>(c, inv, a.inv_thickness[1], a.neg_front[1], a.weight[1], rf, ao);
-            axial2<MODE, 3>(c, inv, a.inv_thickness[2], a.neg_front[2], a.weight[2], rf, ao);
-            axial2<MODE, 4>(c, inv, a.inv_thickness[3], a.neg_front[3], a.weight[3], rf, ao);
-            diag2<MODE, 1>(c, inv, a.inv_thickness[4], a.neg_front[4], a.weight[4], rf, ao);
-            diag2<MODE, 2>(c, inv, a.inv_thickness[5], a.neg_front[5], a.weight[5], rf, ao);
-            diag2<MODE, 3>(c, inv, a.inv_thickness[6], a.neg_front[6], a.weight[6], rf, ao);
-            lshape2<MODE, 1, 2>(c, inv, a.inv_thickness[7], a.neg_front[7], a.weight[7], rf, ao);
-            lshape2<MODE, 1, 3>(c, inv, a.inv_thickness[8], a.neg_front[8], a.weight[8], rf, ao);
-            lshape2<MODE, 1, 4>(c, inv, a.inv_thickness[9], a.neg_front[9], a.weight[9], rf, ao);
-            lshape2<MODE, 2, 3>(c, inv, a.inv_thickness[10], a.neg_front[10], a.weight[10], rf, ao);
-            lshape2<MODE, 2, 4>(c, inv, a.inv_thickness[11], a.neg_front[11], a.weight[11], rf, ao);
-        }
-        // REN:176  lerp(1, ao, gIntensity) -> R8
-        const float2 le = __ffma2_rn(make_float2(a.intensity, a.intensity), __fadd2_rn(ao, make_float2(-1.0f, -1.0f)), make_float2(1.0f, 1.0f));
-        const uint32_t k0 = unorm8_code(le.x);
-        const uint32_t k1 = unorm8_code(le.y);
-        uint8_t *dst = a.occ + (size_t)oy * a.opitch + ox;
-        if (ox + 1 < a.lw) *reinterpret_cast<uint16_t *>(dst) = (uint16_t)(k0 | (k1 << 8));
-        else dst[0] = (uint8_t)k0;
-    }
-#endif
-}
-
+#if !MEAO_REN_BATCH
 // debug view: TiledDepth<k>[slice][j][i] exactly as Downsample1/2 would have written it
 __global__ void synth_tiled_kernel(const float *low, int lw, int lh, int lpitch, int sw, int sh, float pad, __half *out)
 {
@@ -263,9 +141,11 @@ __global__ void synth_tiled_kernel(const float *low, int lw, int lh, int lpitch,
     if (x < lw && y < lh) v = low[(size_t)y * lpitch + x];
     out[((size_t)s * sh + j) * sw + i] = __float2half_rn(v);
 }
+#endif
 
 }  // namespace
 
+#if !MEAO_REN_BATCH
 template <int MODE, bool EXH, int TH>
 static void launch_render_variant(const CUtensorMap &low_map, int t, const RenderArgs &a, dim3 grid, cudaStream_t s)
 {
@@ -314,6 +194,49 @@ cudaError_t preload_render_ao()
     t(synth_tiled_kernel);
     return e;
 }
+#endif
+#else   // render_ao_batch.cu
+template <int MODE, bool EXH, int TH>
+static void launch_render_batch_variant(const CUtensorMap &low_map, int t, const RenderBatchArgs &a, dim3 grid, cudaStream_t s)
+{
+    const size_t smem = (size_t)Geo<MODE, TH>::kSW * Geo<MODE, TH>::kSH * sizeof(float);
+    MEAO_LAUNCH((render_ao_batch_kernel<MODE, EXH, TH>), grid, kThreads, smem, s, low_map, a, t);
+}
+template <int MODE, bool EXH>
+static cudaError_t launch_render_batch_th(const CUtensorMap &low_map, int t, const RenderBatchArgs &b, int gx, int rows, int frames, cudaStream_t s)
+{
+    switch (b.base.tile_h) {
+        case kRenderTileHs[0]: launch_render_batch_variant<MODE, EXH, kRenderTileHs[0]>(low_map, t, b, dim3(gx, ceil_div(rows, kRenderTileHs[0]), frames), s); break;
+        case kRenderTileHs[1]: launch_render_batch_variant<MODE, EXH, kRenderTileHs[1]>(low_map, t, b, dim3(gx, ceil_div(rows, kRenderTileHs[1]), frames), s); break;
+        case kRenderTileHs[2]: launch_render_batch_variant<MODE, EXH, kRenderTileHs[2]>(low_map, t, b, dim3(gx, ceil_div(rows, kRenderTileHs[2]), frames), s); break;
+        default: return cudaErrorInvalidValue;
+    }
+    return cudaGetLastError();
+}
+
+cudaError_t launch_render_ao_batch(const CUtensorMap &low_map3, bool use_tma, const RenderBatchArgs &b, int frames, cudaStream_t s)
+{
+    const RenderArgs &a = b.base;
+    if (a.row1 <= a.row0 || frames < 1) return cudaSuccess;
+    const int ybase = a.row0 & ~3;
+    const int gx = ceil_div(a.lw, kTW), rows = a.row1 - ybase;
+    const int t = use_tma ? 1 : 0;
+    if (!a.wide) return a.exhaustive ? launch_render_batch_th<0, true>(low_map3, t, b, gx, rows, frames, s) : launch_render_batch_th<0, false>(low_map3, t, b, gx, rows, frames, s);
+    return a.exhaustive ? launch_render_batch_th<1, true>(low_map3, t, b, gx, rows, frames, s) : launch_render_batch_th<1, false>(low_map3, t, b, gx, rows, frames, s);
+}
+
+#ifndef MEAO_EMULATE
+cudaError_t preload_render_ao_batch()
+{
+    cudaError_t e = cudaSuccess;
+    auto t = [&](auto k) { if (e == cudaSuccess) e = preload_kernel(k); };
+    t(render_ao_batch_kernel<0, false, 32>); t(render_ao_batch_kernel<0, false, 16>); t(render_ao_batch_kernel<0, false, 8>);
+    t(render_ao_batch_kernel<0, true, 32>); t(render_ao_batch_kernel<0, true, 16>); t(render_ao_batch_kernel<0, true, 8>);
+    t(render_ao_batch_kernel<1, false, 32>); t(render_ao_batch_kernel<1, false, 16>); t(render_ao_batch_kernel<1, false, 8>);
+    t(render_ao_batch_kernel<1, true, 32>); t(render_ao_batch_kernel<1, true, 16>); t(render_ao_batch_kernel<1, true, 8>);
+    return e;
+}
+#endif
 #endif
 
 }  // namespace meao
