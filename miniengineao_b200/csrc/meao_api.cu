@@ -24,6 +24,7 @@
 #include "../../include/meao.h"
 #include "common.cuh"
 #include "kernels.h"
+#include "frame_plan.h"
 
 using namespace meao;
 
@@ -31,9 +32,7 @@ namespace {
 
 thread_local std::string g_create_error;
 
-struct Range { int lo, hi; };   // [lo, hi)
 inline Range clampr(Range r, int n) { Range o{r.lo < 0 ? 0 : r.lo, r.hi > n ? n : r.hi}; if (o.hi < o.lo) o.hi = o.lo; return o; }
-inline int align_up(int x, int a) { return (x + a - 1) / a * a; }
 
 // cuTensorMapEncodeTiled is fetched through the runtime so libmeao.so has no link-time
 // dependency on libcuda (it must load on a machine without a driver for the ABI tests).
@@ -41,49 +40,34 @@ typedef CUresult (*PFN_encodeTiled)(CUtensorMap *, CUtensorMapDataType, cuuint32
                                     const cuuint64_t *, const cuuint32_t *, const cuuint32_t *, CUtensorMapInterleave,
                                     CUtensorMapSwizzle, CUtensorMapL2promotion, CUtensorMapFloatOOBfill);
 
-struct Plan {
-    // Render (per level 1..4) -- AO.cs:660-734
-    float inv_thickness[5][12];
-    float sample_weight[5][12];
-    float inv_slice_dim[5][2];
-    float reject_fadeoff;
-    float intensity;
-    float pad[5];
-    float inv_thickness_wide[5][12];       // the same for a NON-tiled source LowDepth<k> (kernel "main", AO.cs:679)
-    float inv_slice_dim_wide[5][2];
-    // Upsample (per lo level 1..4) -- AO.cs:750-771
-    float inv_low[5][2], inv_high[5][2];
-    float noise_filter_strength[5], step_size[5], blur_tolerance[5], upsample_tolerance[5];
-    float zb[4];
+// The TMA maps of one arena (frame_plan.h map specs); all zero when tma_ok is false.
+struct FrameMaps {
+    bool tma_ok = false;
+    CUtensorMap low_ren[kRenderTileVariants][5];    // LowDepth<k> with the render box of tile height kRenderTileHs[t]
+    CUtensorMap low_wide[kRenderTileVariants][5];   // LowDepth<k> with the wide-render box
+    CUtensorMap low_ups[5];                 // LowDepth<k> with the upsample depth box
+    CUtensorMap ao_ups[2][5];               // [single_scale][k]: LoResAO1 of upsample lo level k (lo_res_ao)
+    CUtensorMap hq_ups[5];                  // HighQuality<k> as LoResAO2 of upsample lo level k
 };
 
 // Batch arena (meao_render_batch): `capacity` frame slots of every intermediate, apart from the single-frame arena so that a
-// batch never disturbs meao_get_buffer / debug views / stage calls / the band flags.  Frame f of a buffer is at ptr + f * slot_bytes.
+// batch never disturbs meao_get_buffer / debug views / stage calls / the band flags.  Frame f of a buffer is at its slot-0
+// pointer + f * slot_bytes; the maps are 3-D (w, h, capacity) with strides (pitch, slot_bytes).
 struct BatchArena {
     void *base = nullptr;
-    size_t bytes = 0, slot_bytes = 0;
+    size_t slot_bytes = 0;
     int capacity = 0;
     int last_frames = 0;                    // frames of the last batch (meao_get_batch_buffer)
     int last_kind = MEAO_DEPTH_RAW_F32;
     uint32_t *tile_ctr = nullptr;           // its own persistent-loop counters: a batch and a single frame never share a word
-    __half *lin = nullptr;
-    float *low[5] = {nullptr};
-    uint8_t *occ[5] = {nullptr}, *comb[4] = {nullptr}, *hq[5] = {nullptr};
-    bool tma_ok = false;
-    // 3-D maps (w, h, capacity), strides (pitch, slot_bytes); same boxes as the single-frame maps
-    CUtensorMap map_low_ren[kRenderTileVariants][5], map_low_wide[kRenderTileVariants][5];
-    CUtensorMap map_low_ups[5], map_ao_ups[5], map_hq_ups[5], map_occ1_ups;
-};
-
-// what the recorders need to know about a batched launch (nullptr: the single-frame path, today's launches)
-struct BatchRun {
-    int frames;
-    long long in_frame_bytes;               // depth stride between frames (W * H * element size)
+    FrameBufs bufs;                         // slot 0
+    FrameMaps maps;
 };
 
 }  // namespace
 
-struct MeaoCtx {
+// Opaque to callers (include/meao.h declares it with default visibility): nothing of it, its constructor included, is exported.
+struct __attribute__((visibility("hidden"))) MeaoCtx {
     int device = 0;
     bool plan_only = false;                 // device < 0: host-side planning only (no CUDA calls at all)
     uint32_t flags = 0;
@@ -99,20 +83,15 @@ struct MeaoCtx {
     bool plan_dirty = true;
     Plan plan;
 
-    int W = 0, H = 0;
-    int lw[7] = {0}, lh[7] = {0};
+    FrameGeom g;                            // W = 0: not sized yet
     // band (global L0 rows) + neighbours
     int band0 = 0, band1 = 0, prev0 = -1, next1 = -1;
 
     // device buffers (natural layout, pitched, global coordinates)
     void *arena = nullptr;
     size_t arena_bytes = 0;
-    __half *lin = nullptr; int lin_pitch = 0;
-    float *low[5] = {nullptr}; int low_pitch[5] = {0};
-    uint8_t *occ[5] = {nullptr}; int occ_pitch[5] = {0};
-    uint8_t *comb[4] = {nullptr};           // same pitch as occ of that level
-    uint8_t *hq[5] = {nullptr};             // HighQuality<k> (kernel "main" output), same pitch as occ of that level
-    uint8_t *result = nullptr; int result_pitch = 0;
+    FrameBufs bufs;                         // the arena's one frame slot
+    uint8_t *result = nullptr;              // the AO texture
     // staging for the host path: two slots so that the H2D copy of frame i+1 overlaps the kernels and the
     // D2H copy of frame i (meao_render_host_async)
     float *depth_stage[2] = {nullptr, nullptr};     // device, W*H each
@@ -122,13 +101,7 @@ struct MeaoCtx {
     cudaEvent_t compute_done = nullptr;
     bool compute_done_valid = false;
 
-    bool tma_ok = false;
-    CUtensorMap map_low_ren[kRenderTileVariants][5];    // LowDepth<k> with the render box of tile height kRenderTileHs[t]
-    CUtensorMap map_low_ups[5];             // LowDepth<k> with the upsample depth box
-    CUtensorMap map_ao_ups[5];              // lo AO of upsample lo level k (Occlusion4 / Combined k)
-    CUtensorMap map_low_wide[kRenderTileVariants][5];   // LowDepth<k> with the wide-render box
-    CUtensorMap map_hq_ups[5];              // HighQuality<k> as LoResAO2 of upsample lo level k
-    CUtensorMap map_occ1_ups;               // Occlusion1 as LoResAO1 of the final upsample (MeaoVariants.single_scale)
+    FrameMaps maps;
 
     // native neighbour exchange (meao_band_export / _connect / _step)
     BandFlags *band_flags = nullptr;        // first 256 bytes of the arena
@@ -182,8 +155,6 @@ int fail(MeaoCtx *c, int code, const char *fmt, ...)
 float mathf_sqrt(float f) { return (float)std::sqrt((double)f); }
 float mathf_pow(float f, float p) { return (float)std::pow((double)f, (double)p); }
 
-float host_f16_round(float x) { return __half2float(__float2half_rn(x)); }
-
 // AO.cs:577-590
 void sample_thickness(float t[12])
 {
@@ -207,19 +178,19 @@ void build_plan(MeaoCtx *c)
     float thick[12];
     sample_thickness(thick);
     for (int k = 1; k <= 4; k++) {
-        const int src_w = c->lw[k + 2], src_h = c->lh[k + 2];
+        const int src_w = c->g.lw[k + 2], src_h = c->g.lh[k + 2];
         const float ScreenspaceDiameter = 10;                                                        // AO.cs:669
         float ThicknessMultiplier = 2 * c->camera.tan_half_fov_h * ScreenspaceDiameter / src_w;     // AO.cs:678
         if (c->variants.single_pass_stereo) ThicknessMultiplier *= 2;                                // AO.cs:680
         float InverseRangeFactor = 1 / ThicknessMultiplier;                                          // AO.cs:683
         for (int i = 0; i < 12; i++) p.inv_thickness[k][i] = InverseRangeFactor / thick[i];          // AO.cs:687-688
         {   // the same recorder fed a non-tiled source (LowDepth<k>): kernel "main"
-            float tm = 2 * c->camera.tan_half_fov_h * ScreenspaceDiameter / c->lw[k];               // AO.cs:678
+            float tm = 2 * c->camera.tan_half_fov_h * ScreenspaceDiameter / c->g.lw[k];               // AO.cs:678
             tm *= 2;                                                                                 // AO.cs:679 (!source.isTiled)
             if (c->variants.single_pass_stereo) tm *= 2;                                             // AO.cs:680
             const float irf = 1 / tm;                                                                // AO.cs:683
             for (int i = 0; i < 12; i++) p.inv_thickness_wide[k][i] = irf / thick[i];
-            p.inv_slice_dim_wide[k][0] = 1.0f / c->lw[k]; p.inv_slice_dim_wide[k][1] = 1.0f / c->lh[k];
+            p.inv_slice_dim_wide[k][0] = 1.0f / c->g.lw[k]; p.inv_slice_dim_wide[k][1] = 1.0f / c->g.lh[k];
         }
         static const float mult[12] = {4, 4, 4, 4, 4, 8, 8, 8, 4, 8, 8, 4};                          // AO.cs:696-707
         float *w = p.sample_weight[k];
@@ -242,7 +213,7 @@ void build_plan(MeaoCtx *c)
     p.intensity = c->params.intensity;                                                               // AO.cs:734
 
     for (int lo = 1; lo <= 4; lo++) {
-        const int lo_w = c->lw[lo], lo_h = c->lh[lo], hi_w = c->lw[lo - 1], hi_h = c->lh[lo - 1];
+        const int lo_w = c->g.lw[lo], lo_h = c->g.lh[lo], hi_w = c->g.lw[lo - 1], hi_h = c->g.lh[lo - 1];
         float stepSize = 1920.0f / lo_w;                                                             // AO.cs:760
         float blurTolerance = 1 - mathf_pow(10, c->params.blur_tolerance) * stepSize;                // AO.cs:761
         blurTolerance *= blurTolerance;                                                              // AO.cs:762
@@ -296,27 +267,38 @@ void free_buffers(MeaoCtx *c)
     c->compute_done_valid = false;
 }
 
-int make_map(MeaoCtx *c, CUtensorMap *m, CUtensorMapDataType dt, int elem, void *base, int w, int h, int pitch_elems, int bw, int bh)
+// frames = 0: a 2-D map (w, h); else a 3-D map (w, h, frames) whose frames are slot_bytes apart, read one frame per box
+bool encode_map(MeaoCtx *c, CUtensorMap *m, const MapSpec &s, int frames, size_t slot_bytes)
 {
-    cuuint64_t dims[2] = {(cuuint64_t)w, (cuuint64_t)h};
-    cuuint64_t strides[1] = {(cuuint64_t)pitch_elems * elem};
-    cuuint32_t box[2] = {(cuuint32_t)bw, (cuuint32_t)bh};
-    cuuint32_t estr[2] = {1, 1};
-    CUresult r = c->encode(m, dt, 2, base, dims, strides, box, estr, CU_TENSOR_MAP_INTERLEAVE_NONE,
-                           CU_TENSOR_MAP_SWIZZLE_NONE, CU_TENSOR_MAP_L2_PROMOTION_L2_128B, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
-    return r == CUDA_SUCCESS ? 0 : -1;
+    const cuuint32_t rank = frames ? 3 : 2;
+    cuuint64_t dims[3] = {(cuuint64_t)s.w, (cuuint64_t)s.h, (cuuint64_t)frames};
+    cuuint64_t strides[2] = {(cuuint64_t)s.pitch_bytes, (cuuint64_t)slot_bytes};
+    cuuint32_t box[3] = {(cuuint32_t)s.bw, (cuuint32_t)s.bh, 1};
+    cuuint32_t estr[3] = {1, 1, 1};
+    CUresult r = c->encode(m, s.elem == 4 ? CU_TENSOR_MAP_DATA_TYPE_FLOAT32 : CU_TENSOR_MAP_DATA_TYPE_UINT8, rank, (void *)s.base, dims,
+                           strides, box, estr, CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_NONE, CU_TENSOR_MAP_L2_PROMOTION_L2_128B,
+                           CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
+    return r == CUDA_SUCCESS;
 }
 
-int make_map3(MeaoCtx *c, CUtensorMap *m, CUtensorMapDataType dt, int elem, void *base, int w, int h, int pitch_elems, int frames,
-              size_t slot_bytes, int bw, int bh)
+void build_maps(MeaoCtx *c, FrameMaps *m, const FrameBufs &b, int frames, size_t slot_bytes)
 {
-    cuuint64_t dims[3] = {(cuuint64_t)w, (cuuint64_t)h, (cuuint64_t)frames};
-    cuuint64_t strides[2] = {(cuuint64_t)pitch_elems * elem, (cuuint64_t)slot_bytes};
-    cuuint32_t box[3] = {(cuuint32_t)bw, (cuuint32_t)bh, 1};
-    cuuint32_t estr[3] = {1, 1, 1};
-    CUresult r = c->encode(m, dt, 3, base, dims, strides, box, estr, CU_TENSOR_MAP_INTERLEAVE_NONE,
-                           CU_TENSOR_MAP_SWIZZLE_NONE, CU_TENSOR_MAP_L2_PROMOTION_L2_128B, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
-    return r == CUDA_SUCCESS ? 0 : -1;
+    *m = FrameMaps{};
+    if (!c->encode) return;
+    const FrameGeom &g = c->g;
+    bool ok = true;
+    for (int k = 1; k <= 4 && ok; k++) {
+        for (int t = 0; t < kRenderTileVariants; t++) {
+            ok &= encode_map(c, &m->low_ren[t][k], render_map(g, b, k, t, false), frames, slot_bytes);
+            ok &= encode_map(c, &m->low_wide[t][k], render_map(g, b, k, t, true), frames, slot_bytes);
+        }
+        ok &= encode_map(c, &m->low_ups[k], ups_depth_map(g, b, k), frames, slot_bytes);
+        for (int single = 0; single < 2; single++)
+            ok &= encode_map(c, &m->ao_ups[single][k], ups_ao_map(g, lo_res_ao(b, k, single), k), frames, slot_bytes);
+        ok &= encode_map(c, &m->hq_ups[k], ups_ao_map(g, b.hq[k], k), frames, slot_bytes);
+    }
+    if (ok) m->tma_ok = true;
+    else *m = FrameMaps{};
 }
 
 // rows of the low level (after clamping) that an upsample producing hi rows [a,b) reads
@@ -339,9 +321,9 @@ BandNeeds compute_needs(const MeaoCtx *c, int b0, int b1)
 {
     BandNeeds n;
     n.need_c[0] = Range{b0, b1};
-    for (int k = 1; k <= 4; k++) n.need_c[k] = ups_lo_rows(n.need_c[k - 1], c->lh[k]);
+    for (int k = 1; k <= 4; k++) n.need_c[k] = ups_lo_rows(n.need_c[k - 1], c->g.lh[k]);
     for (int k = 1; k <= 4; k++) {
-        Range r = ren_low_rows(n.need_c[k], c->lh[k]);
+        Range r = ren_low_rows(n.need_c[k], c->g.lh[k]);
         // the upsample also reads LowDepth<k> on need_c[k] (as lo depth) -- a subset of r
         if (n.need_c[k].lo < r.lo) r.lo = n.need_c[k].lo;
         if (n.need_c[k].hi > r.hi) r.hi = n.need_c[k].hi;
@@ -371,36 +353,20 @@ int setup_band(MeaoCtx *c)
 
 int allocate(MeaoCtx *c)
 {
-    const int W = c->W, H = c->H;
-    for (int l = 0; l < 7; l++) {                         // AO.cs:276-281
-        const int div = 1 << l;
-        c->lw[l] = (W + div - 1) / div;
-        c->lh[l] = (H + div - 1) / div;
-    }
+    c->g = frame_geom(c->g.W, c->g.H);
+    const int W = c->g.W, H = c->g.H;
     c->band0 = 0; c->band1 = H; c->prev0 = -1; c->next1 = -1;
     c->plan_dirty = true;
     if (c->plan_only) return setup_band(c);
     free_buffers(c);
-    // pitches: rows start on 128-byte boundaries
-    c->lin_pitch = align_up(c->lw[0], 64);
-    c->result_pitch = align_up(c->lw[0], 128);
+    const SlotLayout slot = slot_layout(c->g);
     size_t off = 0;
-    auto take = [&](size_t bytes) { size_t o = off; off += (bytes + 255) / 256 * 256; return o; };
-    take(sizeof(BandFlags));            // offset 0 in EVERY context's arena (the neighbours address it through their peer mapping)
-    const size_t o_ctr = take(8 * sizeof(uint32_t));
-    size_t o_lin = take((size_t)c->lin_pitch * c->lh[0] * sizeof(__half));
-    size_t o_res = take((size_t)c->result_pitch * c->lh[0]);
-    size_t o_low[5], o_occ[5], o_comb[4], o_hq[5];
-    for (int k = 1; k <= 4; k++) {
-        c->low_pitch[k] = align_up(c->lw[k], 32);
-        c->occ_pitch[k] = align_up(c->lw[k], 128);
-        o_low[k] = take((size_t)c->low_pitch[k] * c->lh[k] * sizeof(float));
-        o_occ[k] = take((size_t)c->occ_pitch[k] * c->lh[k]);
-        if (k <= 3) o_comb[k] = take((size_t)c->occ_pitch[k] * c->lh[k]);
-        o_hq[k] = take((size_t)c->occ_pitch[k] * c->lh[k]);
-    }
+    take(off, sizeof(BandFlags));       // offset 0 in EVERY context's arena (the neighbours address it through their peer mapping)
+    const size_t o_ctr = take(off, 8 * sizeof(uint32_t));
+    const size_t o_slot = take(off, slot.slot_bytes);
+    const size_t o_res = take(off, (size_t)c->g.result_pitch * c->g.lh[0]);
     size_t o_dst[2], o_ast[2];
-    for (int i = 0; i < 2; i++) { o_dst[i] = take((size_t)W * H * sizeof(float)); o_ast[i] = take((size_t)W * H); }
+    for (int i = 0; i < 2; i++) { o_dst[i] = take(off, (size_t)W * H * sizeof(float)); o_ast[i] = take(off, (size_t)W * H); }
     cudaError_t e = cudaMalloc(&c->arena, off);
     if (e != cudaSuccess) return fail(c, e == cudaErrorMemoryAllocation ? MEAO_ERR_NOMEM : MEAO_ERR_CUDA,
                                       "cudaMalloc(%zu) failed: %s", off, cudaGetErrorString(e));
@@ -415,47 +381,17 @@ int allocate(MeaoCtx *c)
         CUDA_TRY(c, cudaMemcpy(c->band_flags, &init, sizeof init, cudaMemcpyHostToDevice));
         if (c->host_error) *c->host_error = 0;
     }
-    c->lin = (__half *)(b + o_lin);
+    c->bufs = frame_bufs(b + o_slot, slot);
     c->result = (uint8_t *)(b + o_res);
-    for (int k = 1; k <= 4; k++) {
-        c->low[k] = (float *)(b + o_low[k]);
-        c->occ[k] = (uint8_t *)(b + o_occ[k]);
-        if (k <= 3) c->comb[k] = (uint8_t *)(b + o_comb[k]);
-        c->hq[k] = (uint8_t *)(b + o_hq[k]);
-    }
     for (int i = 0; i < 2; i++) { c->depth_stage[i] = (float *)(b + o_dst[i]); c->ao_stage[i] = (uint8_t *)(b + o_ast[i]); }
-
-    c->tma_ok = false;
-    if (c->encode) {
-        bool ok = true;
-        for (int k = 1; k <= 4 && ok; k++) {
-            for (int t = 0; t < kRenderTileVariants; t++) {
-                ok &= make_map(c, &c->map_low_ren[t][k], CU_TENSOR_MAP_DATA_TYPE_FLOAT32, 4, c->low[k], c->lw[k], c->lh[k], c->low_pitch[k], kRenderBoxW, render_box_h(kRenderTileHs[t], false)) == 0;
-                ok &= make_map(c, &c->map_low_wide[t][k], CU_TENSOR_MAP_DATA_TYPE_FLOAT32, 4, c->low[k], c->lw[k], c->lh[k], c->low_pitch[k], kRenderWideBoxW, render_box_h(kRenderTileHs[t], true)) == 0;
-            }
-            ok &= make_map(c, &c->map_low_ups[k], CU_TENSOR_MAP_DATA_TYPE_FLOAT32, 4, c->low[k], c->lw[k], c->lh[k], c->low_pitch[k], kUpsDepthBoxW, kUpsDepthBoxH) == 0;
-            uint8_t *ao = (k == 4) ? c->occ[4] : c->comb[k];
-            ok &= make_map(c, &c->map_ao_ups[k], CU_TENSOR_MAP_DATA_TYPE_UINT8, 1, ao, c->lw[k], c->lh[k], c->occ_pitch[k], kUpsAoBoxW, kUpsAoBoxH) == 0;
-            ok &= make_map(c, &c->map_hq_ups[k], CU_TENSOR_MAP_DATA_TYPE_UINT8, 1, c->hq[k], c->lw[k], c->lh[k], c->occ_pitch[k], kUpsAoBoxW, kUpsAoBoxH) == 0;
-        }
-        ok &= make_map(c, &c->map_occ1_ups, CU_TENSOR_MAP_DATA_TYPE_UINT8, 1, c->occ[1], c->lw[1], c->lh[1], c->occ_pitch[1], kUpsAoBoxW, kUpsAoBoxH) == 0;
-        c->tma_ok = ok;
-    }
-    if (!c->tma_ok) {
-        memset(&c->map_occ1_ups, 0, sizeof c->map_occ1_ups);
-        memset(c->map_low_ren, 0, sizeof c->map_low_ren);
-        memset(c->map_low_ups, 0, sizeof c->map_low_ups);
-        memset(c->map_ao_ups, 0, sizeof c->map_ao_ups);
-        memset(c->map_low_wide, 0, sizeof c->map_low_wide);
-        memset(c->map_hq_ups, 0, sizeof c->map_hq_ups);
-    }
+    build_maps(c, &c->maps, c->bufs, 0, 0);
     return setup_band(c);
 }
 
 int ensure_ready(MeaoCtx *c)
 {
     if (!c) return MEAO_ERR_INVALID;
-    if (c->W <= 0) return fail(c, MEAO_ERR_INVALID, "meao_resize has not been called");
+    if (c->g.W <= 0) return fail(c, MEAO_ERR_INVALID, "meao_resize has not been called");
     if (c->plan_only) return fail(c, MEAO_ERR_CUDA, "plan-only context (device < 0): no CUDA device bound, and libmeao has no CPU fallback");
     CUDA_TRY(c, cudaSetDevice(c->device));
     if (c->plan_dirty) { build_plan(c); c->graphs_stale = true; }
@@ -474,199 +410,90 @@ int reserve_batch(MeaoCtx *c, int frames)
         if (it->first.kind >= 400) { cudaGraphExecDestroy(it->second.exec); it = c->graphs.erase(it); } else ++it;
     }
     free_batch(c);
+    const SlotLayout slot = slot_layout(c->g);
     size_t off = 0;
-    auto take = [&](size_t bytes) { size_t o = off; off += (bytes + 255) / 256 * 256; return o; };
-    const size_t o_lin = take((size_t)c->lin_pitch * c->lh[0] * sizeof(__half));
-    size_t o_low[5], o_occ[5], o_comb[4], o_hq[5];
-    for (int k = 1; k <= 4; k++) {
-        o_low[k] = take((size_t)c->low_pitch[k] * c->lh[k] * sizeof(float));
-        o_occ[k] = take((size_t)c->occ_pitch[k] * c->lh[k]);
-        if (k <= 3) o_comb[k] = take((size_t)c->occ_pitch[k] * c->lh[k]);
-        o_hq[k] = take((size_t)c->occ_pitch[k] * c->lh[k]);
-    }
-    const size_t slot = off;                        // a multiple of 256 bytes
-    const size_t head = 256;                        // persistent-loop tile counters
-    const size_t total = head + slot * (size_t)frames;
-    cudaError_t e = cudaMalloc(&b.base, total);
+    take(off, 8 * sizeof(uint32_t));                // persistent-loop tile counters
+    const size_t o_slot0 = take(off, slot.slot_bytes * (size_t)frames);
+    cudaError_t e = cudaMalloc(&b.base, off);
     if (e != cudaSuccess) {
         b.base = nullptr; cudaGetLastError();
-        return fail(c, e == cudaErrorMemoryAllocation ? MEAO_ERR_NOMEM : MEAO_ERR_CUDA, "batch arena cudaMalloc(%zu) failed: %s", total, cudaGetErrorString(e));
+        return fail(c, e == cudaErrorMemoryAllocation ? MEAO_ERR_NOMEM : MEAO_ERR_CUDA, "batch arena cudaMalloc(%zu) failed: %s", off, cudaGetErrorString(e));
     }
-    CUDA_TRY(c, cudaMemset(b.base, 0, head));
-    b.bytes = total; b.slot_bytes = slot; b.capacity = frames;
-    char *p = (char *)b.base;
-    b.tile_ctr = (uint32_t *)p;
-    p += head;
-    b.lin = (__half *)(p + o_lin);
-    for (int k = 1; k <= 4; k++) {
-        b.low[k] = (float *)(p + o_low[k]);
-        b.occ[k] = (uint8_t *)(p + o_occ[k]);
-        if (k <= 3) b.comb[k] = (uint8_t *)(p + o_comb[k]);
-        b.hq[k] = (uint8_t *)(p + o_hq[k]);
-    }
-    b.tma_ok = false;
-    if (c->encode) {
-        bool ok = true;
-        for (int k = 1; k <= 4 && ok; k++) {
-            for (int t = 0; t < kRenderTileVariants; t++) {
-                ok &= make_map3(c, &b.map_low_ren[t][k], CU_TENSOR_MAP_DATA_TYPE_FLOAT32, 4, b.low[k], c->lw[k], c->lh[k], c->low_pitch[k], frames, slot, kRenderBoxW, render_box_h(kRenderTileHs[t], false)) == 0;
-                ok &= make_map3(c, &b.map_low_wide[t][k], CU_TENSOR_MAP_DATA_TYPE_FLOAT32, 4, b.low[k], c->lw[k], c->lh[k], c->low_pitch[k], frames, slot, kRenderWideBoxW, render_box_h(kRenderTileHs[t], true)) == 0;
-            }
-            ok &= make_map3(c, &b.map_low_ups[k], CU_TENSOR_MAP_DATA_TYPE_FLOAT32, 4, b.low[k], c->lw[k], c->lh[k], c->low_pitch[k], frames, slot, kUpsDepthBoxW, kUpsDepthBoxH) == 0;
-            uint8_t *ao = (k == 4) ? b.occ[4] : b.comb[k];
-            ok &= make_map3(c, &b.map_ao_ups[k], CU_TENSOR_MAP_DATA_TYPE_UINT8, 1, ao, c->lw[k], c->lh[k], c->occ_pitch[k], frames, slot, kUpsAoBoxW, kUpsAoBoxH) == 0;
-            ok &= make_map3(c, &b.map_hq_ups[k], CU_TENSOR_MAP_DATA_TYPE_UINT8, 1, b.hq[k], c->lw[k], c->lh[k], c->occ_pitch[k], frames, slot, kUpsAoBoxW, kUpsAoBoxH) == 0;
-        }
-        ok &= make_map3(c, &b.map_occ1_ups, CU_TENSOR_MAP_DATA_TYPE_UINT8, 1, b.occ[1], c->lw[1], c->lh[1], c->occ_pitch[1], frames, slot, kUpsAoBoxW, kUpsAoBoxH) == 0;
-        b.tma_ok = ok;
-    }
+    CUDA_TRY(c, cudaMemset(b.base, 0, o_slot0));
+    b.slot_bytes = slot.slot_bytes; b.capacity = frames;
+    b.tile_ctr = (uint32_t *)b.base;
+    b.bufs = frame_bufs((char *)b.base + o_slot0, slot);
+    build_maps(c, &b.maps, b.bufs, frames, slot.slot_bytes);
     return 0;
 }
 
 struct NvtxRange { explicit NvtxRange(const char *n) { nvtxRangePushA(n); } ~NvtxRange() { nvtxRangePop(); } };
 
-// Tile-height variant (index into kRenderTileHs = {32, 16, 8}) of a render launch.  The big levels keep the 64 x 32 tile
-// (least apron overhead: throughput); a level whose grid would not even put one CTA on every SM is latency-bound -- one
-// CTA's serial time IS the kernel time -- so it takes the tallest tile that still gives >= 148 CTAs, else 64 x 8.
-// (Measured at 4K: level 2, 255 CTAs of 64 x 32, is FASTER with the big tile -- 14.0 vs 15.7 us -- levels 3 / 4 gain ~0.5 us.)
-int render_tile_variant(const MeaoCtx *c, int k, int rows, int frames = 1)
+// render_tile_variant, unless MEAO_REN_TILE (tuning aid: 0 / 1 / 2) forces a variant for every level
+int render_tile(const MeaoCtx *c, int k, int frames)
 {
-    const char *force = getenv("MEAO_REN_TILE");               // tuning aid: 0 / 1 / 2 forces a variant for every level
+    const char *force = getenv("MEAO_REN_TILE");
     if (force && force[0] >= '0' && force[0] < '0' + kRenderTileVariants) return force[0] - '0';
-    for (int t = 0; t < kRenderTileVariants; t++) {
-        const long long ctas = (long long)((c->lw[k] + 63) / 64) * ((rows + kRenderTileHs[t] - 1) / kRenderTileHs[t]) * frames;   // a batch: all its frames
-        if (ctas >= 148) return t;
-    }
-    return kRenderTileVariants - 1;
+    return render_tile_variant(c->g.lw[k], c->need_c[k], frames);
 }
 
 // ---- the three recorders ---------------------------------------------------------------------
+// batch == nullptr: one frame in the context's arena; otherwise every launch covers the batch's frames in the batch arena.
+
+struct ArenaRef { const FrameBufs &bufs; const FrameMaps &maps; uint32_t *tile_ctr; };
+ArenaRef arena_of(const MeaoCtx *c, const BatchRun *batch)
+{
+    return batch ? ArenaRef{c->batch.bufs, c->batch.maps, c->batch.tile_ctr} : ArenaRef{c->bufs, c->maps, c->tile_ctr};
+}
 
 // PushDownsampleCommands, AO.cs:604-658
 int record_downsample(MeaoCtx *c, const void *depth, int kind, cudaStream_t s, const BatchRun *batch = nullptr)
 {
     if (kind < MEAO_DEPTH_RAW_F32 || kind > MEAO_DEPTH_RAW_D24S8) return fail(c, MEAO_ERR_INVALID, "bad depth kind %d", kind);
     NvtxRange nv("meao::prepare_depth");
-    PrepareArgs a{};
-    a.depth = depth;
-    a.in_format = (kind == MEAO_DEPTH_RAW_D16_UNORM) ? 1 : (kind == MEAO_DEPTH_RAW_D24S8 ? 2 : 0);
-    a.W = c->W; a.H = c->H;
-    a.depth_row0 = c->band0;
-    a.row0 = c->band0; a.row1 = c->band1;
-    a.lin = c->lin; a.lin_pitch = c->lin_pitch;
-    for (int k = 1; k <= 4; k++) { a.low[k - 1] = c->low[k]; a.low_pitch[k - 1] = c->low_pitch[k]; }
-    a.zbx = c->plan.zb[0]; a.zby = c->plan.zb[1];
-    a.raw = (kind != MEAO_DEPTH_LINEAR_F32);
-    a.reversed_z = c->camera.reversed_z;
-    a.vec_ok = (((uintptr_t)depth & 15) == 0) && (c->W % (a.in_format == 1 ? 8 : 4) == 0);
+    const PrepareArgs a = prepare_args(c->g, arena_of(c, batch).bufs, c->plan, depth, depth_in_format(kind), kind != MEAO_DEPTH_LINEAR_F32,
+                                       c->camera.reversed_z, Range{c->band0, c->band1}, batch);
     if (batch) {
-        const BatchArena &b = c->batch;
-        a.lin = b.lin;
-        for (int k = 1; k <= 4; k++) a.low[k - 1] = b.low[k];
-        a.vec_ok = a.vec_ok && (batch->in_frame_bytes % 16 == 0);     // every frame's base stays 16-byte aligned
         c->batch.last_kind = kind;
-        CUDA_TRY(c, launch_prepare_depth_batch(PrepareBatchArgs{a, batch->in_frame_bytes, (long long)b.slot_bytes}, batch->frames, s));
-        c->launches++;
-        return 0;
+        CUDA_TRY(c, launch_prepare_depth_batch(PrepareBatchArgs{a, batch->in_frame_bytes, batch->slot_bytes}, batch->frames, s));
+    } else {
+        c->last_kind = kind;
+        CUDA_TRY(c, launch_prepare_depth(a, s));
     }
-    c->last_kind = kind;
-    CUDA_TRY(c, launch_prepare_depth(a, s));
     c->launches++;
     return 0;
 }
 
-// PushRenderCommands, AO.cs:660-748.  wide = false: the call AmbientOcclusion.cs makes (tiled source, kernel main_interleaved);
-// wide = true: the same recorder for the non-tiled source LowDepth<k> (kernel main) -> HighQuality<k>.
+// PushRenderCommands, AO.cs:660-748 (frame_plan.h render_args)
 int record_render(MeaoCtx *c, int k, int kind, cudaStream_t s, bool wide = false, const BatchRun *batch = nullptr)
 {
-    static const int idx_checker[7] = {1, 3, 4, 8, 11, 6, 10};                       // Render.compute:162-168 table slots, call order
-    static const int idx_exh[12] = {0, 1, 2, 3, 4, 8, 11, 5, 6, 7, 9, 10};           // Render.compute:148-159
-    const bool exh = c->variants.sample_exhaustively != 0;
-    const int n = exh ? 12 : 7;
-    const int *idx = exh ? idx_exh : idx_checker;
     NvtxRange nv(wide ? "meao::render_ao_wide" : "meao::render_ao");
-    RenderArgs a{};
-    a.low = c->low[k]; a.lw = c->lw[k]; a.lh = c->lh[k]; a.lpitch = c->low_pitch[k];
-    a.occ = wide ? c->hq[k] : c->occ[k]; a.opitch = c->occ_pitch[k];
-    a.sw = c->lw[k + 2]; a.sh = c->lh[k + 2];
-    a.pad = host_f16_round((kind != MEAO_DEPTH_LINEAR_F32) ? c->plan.pad[k] : 0.0f);
-    const float *it = wide ? c->plan.inv_thickness_wide[k] : c->plan.inv_thickness[k];
-    for (int i = 0; i < n; i++) {
-        a.inv_thickness[i] = it[idx[i]];
-        a.neg_front[i] = -(a.inv_thickness[i] - 0.5f);                                               // Render.compute:85
-        a.weight[i] = c->plan.sample_weight[k][idx[i]];
-    }
-    a.reject_fadeoff = c->plan.reject_fadeoff;
-    a.intensity = c->plan.intensity;
-    a.row0 = c->need_c[k].lo; a.row1 = c->need_c[k].hi;
-    a.wide = wide ? 1 : 0;
-    a.exhaustive = exh ? 1 : 0;
-    const int tv = render_tile_variant(c, k, a.row1 - (a.row0 & ~3), batch ? batch->frames : 1);
-    a.tile_h = kRenderTileHs[tv];
-    if (batch) {
-        const BatchArena &b = c->batch;
-        a.low = b.low[k]; a.occ = wide ? b.hq[k] : b.occ[k];
-        CUDA_TRY(c, launch_render_ao_batch(wide ? b.map_low_wide[tv][k] : b.map_low_ren[tv][k], b.tma_ok, RenderBatchArgs{a, (long long)b.slot_bytes}, batch->frames, s));
-        c->launches++;
-        return 0;
-    }
-    CUDA_TRY(c, launch_render_ao(wide ? c->map_low_wide[tv][k] : c->map_low_ren[tv][k], c->tma_ok, a, s));
+    const ArenaRef ar = arena_of(c, batch);
+    const int tv = render_tile(c, k, batch ? batch->frames : 1);
+    const RenderArgs a = render_args(c->g, ar.bufs, c->plan, k, wide, c->variants.sample_exhaustively != 0, kind != MEAO_DEPTH_LINEAR_F32,
+                                     c->need_c[k], tv);
+    const CUtensorMap &map = wide ? ar.maps.low_wide[tv][k] : ar.maps.low_ren[tv][k];
+    if (batch) CUDA_TRY(c, launch_render_ao_batch(map, ar.maps.tma_ok, RenderBatchArgs{a, batch->slot_bytes}, batch->frames, s));
+    else CUDA_TRY(c, launch_render_ao(map, ar.maps.tma_ok, a, s));
     c->launches++;
     return 0;
 }
-inline bool hq_level(const MeaoCtx *c, int k) { return ((c->variants.high_quality_mask >> (k - 1)) & 1) != 0; }
 
-// PushUpsampleCommands with the wiring of AO.cs:528-531
+// PushUpsampleCommands with the wiring of AO.cs:528-531 (frame_plan.h upsample_args)
 int record_upsample(MeaoCtx *c, int lo, void *ao_out, cudaStream_t s, const BatchRun *batch = nullptr)
 {
-    const int hi = lo - 1;
     NvtxRange nv("meao::blur_upsample");
-    const bool single = c->variants.single_scale != 0 && lo == 1;      // LoResAO1 = Occlusion1: no coarser level contributes
-    UpsampleArgs a{};
-    a.lo_depth = c->low[lo]; a.low = c->lw[lo]; a.loh = c->lh[lo]; a.lo_dpitch = c->low_pitch[lo];
-    a.lo_ao = single ? c->occ[1] : (lo == 4) ? c->occ[4] : c->comb[lo]; a.lo_apitch = c->occ_pitch[lo];
-    if (hi == 0) { a.hi_depth = c->lin; a.hi_is_half = 1; a.hi_dpitch = c->lin_pitch; a.hi_ao = nullptr; a.hi_apitch = 0; }
-    else { a.hi_depth = c->low[hi]; a.hi_is_half = 0; a.hi_dpitch = c->low_pitch[hi]; a.hi_ao = c->occ[hi]; a.hi_apitch = c->occ_pitch[hi]; }
-    if (hi == 0) {
-        if (ao_out) { a.out = (uint8_t *)ao_out; a.out_pitch = c->W; a.out_row_origin = c->band0; }
-        else { a.out = c->result; a.out_pitch = c->result_pitch; a.out_row_origin = 0; }
-        if (!batch) c->last_out = ao_out;
-    } else { a.out = c->comb[hi]; a.out_pitch = c->occ_pitch[hi]; a.out_row_origin = 0; }
-    a.out_vec_ok = (((uintptr_t)a.out & 7) == 0) && (a.out_pitch % 8 == 0);
-    a.hiw = c->lw[hi]; a.hih = c->lh[hi];
-    a.noise_filter_strength = c->plan.noise_filter_strength[lo];
-    a.step_size = c->plan.step_size[lo];
-    a.blur_tolerance = c->plan.blur_tolerance[lo];
-    a.upsample_tolerance = c->plan.upsample_tolerance[lo];
-    {
-        auto safe = [](float x) { return x >= 8.673617379884035e-19f && x < 1152921504606846976.0f; };
-        a.fast_div_ok = safe(a.upsample_tolerance) && safe(a.noise_filter_strength);
-#if MEAO_UPS_STATIC_GUARD || MEAO_UPS_V2
-        // 2^-55, 2^-52, 2^59: with these bounds total / num of the final division are provably inside the fast-division range
-        a.fast_div_ok = a.fast_div_ok && a.upsample_tolerance >= 2.7755575615628914e-17f &&
-                        a.noise_filter_strength >= 2.220446049250313e-16f && a.noise_filter_strength < 288230376151711744.0f;
-#endif
-    }
-    a.row0 = c->need_c[hi].lo; a.row1 = c->need_c[hi].hi;
-    a.tile_ctr = c->tile_ctr + 2 * (lo - 1);
-    const uint8_t *lo_ao2 = hq_level(c, lo) ? c->hq[lo] : nullptr;                   // kernels main_premin / main_premin_blendout
+    const ArenaRef ar = arena_of(c, batch);
+    const UpsamplePreminArgs pa = upsample_args(c->g, ar.bufs, c->plan, c->variants, lo, c->need_c[lo - 1], (uint8_t *)ao_out, c->result,
+                                                c->band0, ar.tile_ctr, batch);
+    const CUtensorMap &ao_map = ar.maps.ao_ups[c->variants.single_scale != 0][lo];
     if (batch) {
-        const BatchArena &b = c->batch;
-        a.lo_depth = b.low[lo];
-        a.lo_ao = single ? b.occ[1] : (lo == 4) ? b.occ[4] : b.comb[lo];
-        if (hi == 0) a.hi_depth = b.lin;
-        else { a.hi_depth = b.low[hi]; a.hi_ao = b.occ[hi]; }
-        long long out_frame_bytes = (long long)b.slot_bytes;
-        if (hi == 0) { a.out = (uint8_t *)ao_out; a.out_pitch = c->W; a.out_row_origin = 0; out_frame_bytes = (long long)c->W * c->H; }
-        else a.out = b.comb[hi];
-        a.out_vec_ok = (((uintptr_t)a.out & 7) == 0) && (a.out_pitch % 8 == 0) && (out_frame_bytes % 8 == 0);
-        a.tile_ctr = b.tile_ctr + 2 * (lo - 1);
-        UpsampleBatchArgs ba{UpsamplePreminArgs{a, hq_level(c, lo) ? b.hq[lo] : nullptr, c->occ_pitch[lo]}, (long long)b.slot_bytes, out_frame_bytes, batch->frames, 0};
-        CUDA_TRY(c, launch_blur_upsample_batch(b.map_low_ups[lo], single ? b.map_occ1_ups : b.map_ao_ups[lo], &b.map_hq_ups[lo], b.tma_ok, ba, s));
-        c->launches++;
-        return 0;
+        const UpsampleBatchArgs ba{pa, batch->slot_bytes, ups_out_frame_bytes(c->g, lo, *batch), batch->frames, 0};
+        CUDA_TRY(c, launch_blur_upsample_batch(ar.maps.low_ups[lo], ao_map, &ar.maps.hq_ups[lo], ar.maps.tma_ok, ba, s));
+    } else {
+        if (lo == 1) c->last_out = ao_out;
+        CUDA_TRY(c, launch_blur_upsample(ar.maps.low_ups[lo], ao_map, &ar.maps.hq_ups[lo], ar.maps.tma_ok, pa.base, pa.lo_ao2, pa.lo_a2pitch, s));
     }
-    CUDA_TRY(c, launch_blur_upsample(c->map_low_ups[lo], single ? c->map_occ1_ups : c->map_ao_ups[lo], &c->map_hq_ups[lo], c->tma_ok, a, lo_ao2, c->occ_pitch[lo], s));
     c->launches++;
     return 0;
 }
@@ -699,15 +526,15 @@ int record_frame_dag(MeaoCtx *c, const void *depth, int kind, void *ao_out, cuda
     CUDA_TRY(c, cudaStreamWaitEvent(b3, c->ev[0], 0));
     // the optional high-quality render of a level (kernel "main") rides on the branch of that level's interleaved render
     { PdlScope p(pdl >= 1 && !after_exchange); if ((rc = record_render(c, 1, kind, s, false, batch))) return rc; }
-    { PdlScope p(pdl >= 1); if (hq_level(c, 1) && (rc = record_render(c, 1, kind, s, true, batch))) return rc; }
+    { PdlScope p(pdl >= 1); if (hq_level(c->variants, 1) && (rc = record_render(c, 1, kind, s, true, batch))) return rc; }
     if ((rc = record_render(c, 2, kind, b1, false, batch))) return rc;
-    { PdlScope p(pdl >= 1); if (hq_level(c, 2) && (rc = record_render(c, 2, kind, b1, true, batch))) return rc; }
+    { PdlScope p(pdl >= 1); if (hq_level(c->variants, 2) && (rc = record_render(c, 2, kind, b1, true, batch))) return rc; }
     CUDA_TRY(c, cudaEventRecord(c->ev[1], b1));
     if ((rc = record_render(c, 3, kind, b2, false, batch))) return rc;
-    { PdlScope p(pdl >= 1); if (hq_level(c, 3) && (rc = record_render(c, 3, kind, b2, true, batch))) return rc; }
+    { PdlScope p(pdl >= 1); if (hq_level(c->variants, 3) && (rc = record_render(c, 3, kind, b2, true, batch))) return rc; }
     CUDA_TRY(c, cudaEventRecord(c->ev[2], b2));
     if ((rc = record_render(c, 4, kind, b3, false, batch))) return rc;
-    { PdlScope p(pdl >= 1); if (hq_level(c, 4) && (rc = record_render(c, 4, kind, b3, true, batch))) return rc; }
+    { PdlScope p(pdl >= 1); if (hq_level(c->variants, 4) && (rc = record_render(c, 4, kind, b3, true, batch))) return rc; }
     CUDA_TRY(c, cudaStreamWaitEvent(b3, c->ev[2], 0));
     { PdlScope p(pdl >= 2); if ((rc = record_upsample(c, 4, nullptr, b3, batch))) return rc; }
     CUDA_TRY(c, cudaStreamWaitEvent(b3, c->ev[1], 0));
@@ -736,7 +563,7 @@ int record_frame(MeaoCtx *c, const void *depth, int kind, void *ao_out, cudaStre
     names.push_back("prepare_depth"); mark();
     const int kmax = c->variants.single_scale ? 1 : 4;       // single-scale: Render level 1 + the final-style Upsample only
     for (int k = 1; k <= kmax; k++) { for (int r = 0; r < reps && !rc; r++) rc = record_render(c, k, kind, s, false, batch); if (rc) return rc; names.push_back(ren_names[k]); mark(); }
-    for (int k = 1; k <= kmax; k++) if (hq_level(c, k)) { for (int r = 0; r < reps && !rc; r++) rc = record_render(c, k, kind, s, true, batch); if (rc) return rc; names.push_back(hq_names[k]); mark(); }
+    for (int k = 1; k <= kmax; k++) if (hq_level(c->variants, k)) { for (int r = 0; r < reps && !rc; r++) rc = record_render(c, k, kind, s, true, batch); if (rc) return rc; names.push_back(hq_names[k]); mark(); }
     for (int lo = kmax; lo >= 1; lo--) { for (int r = 0; r < reps && !rc; r++) rc = record_upsample(c, lo, lo == 1 ? ao_out : nullptr, s, batch); if (rc) return rc; names.push_back(ups_names[lo]); mark(); }
     if (profile) {
         CUDA_TRY(c, cudaStreamSynchronize(s));
@@ -750,31 +577,38 @@ int record_frame(MeaoCtx *c, const void *depth, int kind, void *ao_out, cudaStre
     return 0;
 }
 
-int buffer_info(const MeaoCtx *c, int id, int *lvl, int *slices, int *elem)
+// Copies buffer view v between the device and the host; a TiledDepth view (to the host only) is synthesised from LowDepth<k>
+// with the padding texels of ingest `kind`.  Synchronous: a debug path.
+int transfer_view(MeaoCtx *c, const BufferView &v, int kind, void *host, bool to_host)
 {
-    if (id == 1) { *lvl = 0; *slices = 1; *elem = 2; }
-    else if (id >= 2 && id <= 5) { *lvl = id - 1; *slices = 1; *elem = 4; }
-    else if (id >= 6 && id <= 9) { *lvl = id - 5 + 2; *slices = 16; *elem = 2; }
-    else if (id >= 10 && id <= 13) { *lvl = id - 9; *slices = 1; *elem = 1; }
-    else if (id >= 14 && id <= 16) { *lvl = id - 13; *slices = 1; *elem = 1; }
-    else if (id == 17) { *lvl = 0; *slices = 1; *elem = 1; }
-    else if (id >= 18 && id <= 21) { *lvl = id - 17; *slices = 1; *elem = 1; }      // HighQuality1..4 (extension)
-    else return -1;
-    (void)c;
-    return 0;
+    if (v.slices == 16) {
+        const int k = v.level;
+        __half *tmp = nullptr;
+        CUDA_TRY(c, cudaMalloc(&tmp, v.bytes()));
+        cudaError_t e = launch_synth_tiled((const float *)v.ptr, c->g.lw[k], c->g.lh[k], c->g.low_pitch[k], v.w, v.h,
+                                           atlas_pad(c->plan, k, kind != MEAO_DEPTH_LINEAR_F32), tmp, c->stream);
+        if (e == cudaSuccess) e = cudaMemcpyAsync(host, tmp, v.bytes(), cudaMemcpyDeviceToHost, c->stream);
+        if (e == cudaSuccess) e = cudaStreamSynchronize(c->stream);
+        cudaFree(tmp);
+        if (e != cudaSuccess) return fail(c, MEAO_ERR_CUDA, "tiled view: %s", cudaGetErrorString(e));
+        return MEAO_OK;
+    }
+    const size_t wb = (size_t)v.w * v.elem;
+    if (to_host) CUDA_TRY(c, cudaMemcpy2DAsync(host, wb, v.ptr, v.pitch_bytes, wb, v.h, cudaMemcpyDeviceToHost, c->stream));
+    else CUDA_TRY(c, cudaMemcpy2DAsync(v.ptr, v.pitch_bytes, host, wb, wb, v.h, cudaMemcpyHostToDevice, c->stream));
+    CUDA_TRY(c, cudaStreamSynchronize(c->stream));
+    return MEAO_OK;
 }
 
-// device pointer + pitch (bytes) of a non-tiled buffer
-int buffer_ptr(MeaoCtx *c, int id, void **p, size_t *pitch_bytes)
+// The last frame wrote the AO texture straight into the caller's buffer: regenerate the context's own copy (buffer 17) from the
+// still resident Combined1 / LowDepth1 / LinearDepth with the same kernel.
+int refresh_result(MeaoCtx *c, cudaStream_t s)
 {
-    if (id == 1) { *p = c->lin; *pitch_bytes = (size_t)c->lin_pitch * 2; }
-    else if (id >= 2 && id <= 5) { *p = c->low[id - 1]; *pitch_bytes = (size_t)c->low_pitch[id - 1] * 4; }
-    else if (id >= 10 && id <= 13) { *p = c->occ[id - 9]; *pitch_bytes = c->occ_pitch[id - 9]; }
-    else if (id >= 14 && id <= 16) { *p = c->comb[id - 13]; *pitch_bytes = c->occ_pitch[id - 13]; }
-    else if (id == 17) { *p = c->result; *pitch_bytes = c->result_pitch; }
-    else if (id >= 18 && id <= 21) { *p = c->hq[id - 17]; *pitch_bytes = c->occ_pitch[id - 17]; }
-    else return -1;
-    return 0;
+    if (!c->last_out) return 0;
+    const int64_t before = c->launches;
+    const int rc = record_upsample(c, 1, nullptr, s);
+    c->launches = before;
+    return rc;
 }
 
 std::mutex g_event_mutex;
@@ -949,25 +783,25 @@ int meao_resize(MeaoCtx *c, int32_t w, int32_t h)
 {
     if (!c) return MEAO_ERR_INVALID;
     if (w <= 0 || h <= 0 || w > 32768 || h > 32768) return fail(c, MEAO_ERR_INVALID, "bad size %dx%d", w, h);
-    if (w == c->W && h == c->H && (c->arena || c->plan_only)) return 0;       // RTHandle.CheckBaseDimensions, AO.cs:145-148
+    if (w == c->g.W && h == c->g.H && (c->arena || c->plan_only)) return 0;       // RTHandle.CheckBaseDimensions, AO.cs:145-148
     if (!c->plan_only) {
         CUDA_TRY(c, cudaSetDevice(c->device));
         CUDA_TRY(c, cudaStreamSynchronize(c->stream));
     }
-    c->W = w; c->H = h;
+    c->g.W = w; c->g.H = h;
     int rc = allocate(c);
-    if (rc) { c->W = c->H = 0; return rc; }
+    if (rc) { c->g.W = c->g.H = 0; return rc; }
     return 1;
 }
 
 int meao_set_row_band(MeaoCtx *c, int32_t row0, int32_t row1, int32_t prev_row0, int32_t next_row1)
 {
-    if (!c || c->W <= 0) return MEAO_ERR_INVALID;
-    if (row0 < 0 || row1 > c->H || row0 >= row1 || (row0 % 16) || ((row1 % 16) && row1 != c->H))
-        return fail(c, MEAO_ERR_INVALID, "band [%d,%d) must be 16-row aligned inside [0,%d)", row0, row1, c->H);
-    if ((prev_row0 >= 0 && (prev_row0 % 16 || prev_row0 >= row0)) || (next_row1 >= 0 && (next_row1 <= row1 || next_row1 > c->H)))
+    if (!c || c->g.W <= 0) return MEAO_ERR_INVALID;
+    if (row0 < 0 || row1 > c->g.H || row0 >= row1 || (row0 % 16) || ((row1 % 16) && row1 != c->g.H))
+        return fail(c, MEAO_ERR_INVALID, "band [%d,%d) must be 16-row aligned inside [0,%d)", row0, row1, c->g.H);
+    if ((prev_row0 >= 0 && (prev_row0 % 16 || prev_row0 >= row0)) || (next_row1 >= 0 && (next_row1 <= row1 || next_row1 > c->g.H)))
         return fail(c, MEAO_ERR_INVALID, "bad neighbour extents");
-    if ((row0 > 0) != (prev_row0 >= 0) || (row1 < c->H) != (next_row1 >= 0))
+    if ((row0 > 0) != (prev_row0 >= 0) || (row1 < c->g.H) != (next_row1 >= 0))
         return fail(c, MEAO_ERR_INVALID, "neighbour extents must be given exactly where the band is interior");
     // validate against temporaries; the context keeps its old band when the new one is refused
     {
@@ -1013,23 +847,23 @@ static void halo_ranges(MeaoCtx *c, int side, bool send, Range out[5])
 
 static int64_t halo_size(MeaoCtx *c, int side, bool send)
 {
-    if (!c || c->W <= 0 || (side != 0 && side != 1)) return MEAO_ERR_INVALID;
+    if (!c || c->g.W <= 0 || (side != 0 && side != 1)) return MEAO_ERR_INVALID;
     Range r[5]; halo_ranges(c, side, send, r);
     int64_t bytes = 0;
-    for (int k = 1; k <= 4; k++) bytes += (int64_t)(r[k].hi - r[k].lo) * c->lw[k] * 4;
+    for (int k = 1; k <= 4; k++) bytes += (int64_t)(r[k].hi - r[k].lo) * c->g.lw[k] * 4;
     return bytes;
 }
 int64_t meao_halo_bytes(MeaoCtx *c, int32_t side) { return halo_size(c, side, true); }
 int meao_halo_rows(MeaoCtx *c, int32_t side, int32_t send, int32_t out8[8])
 {
-    if (!c || c->W <= 0 || (side != 0 && side != 1) || !out8) return MEAO_ERR_INVALID;
+    if (!c || c->g.W <= 0 || (side != 0 && side != 1) || !out8) return MEAO_ERR_INVALID;
     Range r[5]; halo_ranges(c, side, send != 0, r);
     for (int k = 1; k <= 4; k++) { out8[2 * (k - 1)] = r[k].lo; out8[2 * (k - 1) + 1] = r[k].hi; }
     return MEAO_OK;
 }
 int meao_band_rows(MeaoCtx *c, int32_t out30[30])
 {
-    if (!c || c->W <= 0 || !out30) return MEAO_ERR_INVALID;
+    if (!c || c->g.W <= 0 || !out30) return MEAO_ERR_INVALID;
     for (int k = 0; k <= 4; k++) {
         out30[2 * k] = c->need_c[k].lo; out30[2 * k + 1] = c->need_c[k].hi;
         out30[10 + 2 * k] = c->need_low[k].lo; out30[10 + 2 * k + 1] = c->need_low[k].hi;
@@ -1049,8 +883,8 @@ static int halo_copy(MeaoCtx *c, int side, void *packed, bool pack, void *stream
     for (int k = 1; k <= 4; k++) {
         const int rows = r[k].hi - r[k].lo;
         if (rows <= 0) continue;
-        const size_t wb = (size_t)c->lw[k] * 4, pb = (size_t)c->low_pitch[k] * 4;
-        char *buf = (char *)(c->low[k] + (size_t)r[k].lo * c->low_pitch[k]);
+        const size_t wb = (size_t)c->g.lw[k] * 4, pb = (size_t)c->g.low_pitch[k] * 4;
+        char *buf = (char *)(c->bufs.low[k] + (size_t)r[k].lo * c->g.low_pitch[k]);
         if (pack) CUDA_TRY(c, cudaMemcpy2DAsync(p, wb, buf, pb, wb, rows, cudaMemcpyDeviceToDevice, s));
         else      CUDA_TRY(c, cudaMemcpy2DAsync(buf, pb, p, wb, wb, rows, cudaMemcpyDeviceToDevice, s));
         p += wb * rows;
@@ -1073,7 +907,7 @@ int meao_render_band_finish(MeaoCtx *c, void *ao_out, void *stream)
     cudaStream_t s = (cudaStream_t)stream;
     const int kind = c->last_kind;
     for (int k = 1; k <= 4; k++) if ((rc = record_render(c, k, kind, s))) return rc;
-    for (int k = 1; k <= 4; k++) if (hq_level(c, k) && (rc = record_render(c, k, kind, s, true))) return rc;
+    for (int k = 1; k <= 4; k++) if (hq_level(c->variants, k) && (rc = record_render(c, k, kind, s, true))) return rc;
     for (int lo = 4; lo >= 1; lo--) if ((rc = record_upsample(c, lo, lo == 1 ? ao_out : nullptr, s))) return rc;
     return MEAO_OK;
 }
@@ -1089,11 +923,11 @@ static int halo_kernel(MeaoCtx *c, void *up, void *down, bool pack, cudaStream_t
         for (int k = 1; k <= 4; k++) {
             const int rows = r[k].hi - r[k].lo;
             if (rows <= 0) continue;
-            float *buf = c->low[k] + (size_t)r[k].lo * c->low_pitch[k];
+            float *buf = c->bufs.low[k] + (size_t)r[k].lo * c->g.low_pitch[k];
             HaloSeg &g = a.seg[a.nseg++];
-            if (pack) g = HaloSeg{buf, p, c->low_pitch[k], c->lw[k], c->lw[k], rows};
-            else      g = HaloSeg{p, buf, c->lw[k], c->low_pitch[k], c->lw[k], rows};
-            p += (size_t)rows * c->lw[k];
+            if (pack) g = HaloSeg{buf, p, c->g.low_pitch[k], c->g.lw[k], c->g.lw[k], rows};
+            else      g = HaloSeg{p, buf, c->g.lw[k], c->g.low_pitch[k], c->g.lw[k], rows};
+            p += (size_t)rows * c->g.lw[k];
         }
     }
     CUDA_TRY(c, launch_halo_copy(a, s));
@@ -1217,7 +1051,7 @@ int meao_band_export(MeaoCtx *c, MeaoPeerHandle *out)
     int rc = ensure_ready(c); if (rc) return rc;
     if (!out) return fail(c, MEAO_ERR_INVALID, "out is NULL");
     PeerHandlePod h{};
-    h.magic = kPeerMagic; h.device = c->device; h.pid = (int64_t)getpid(); h.W = c->W; h.H = c->H;
+    h.magic = kPeerMagic; h.device = c->device; h.pid = (int64_t)getpid(); h.W = c->g.W; h.H = c->g.H;
     h.arena_bytes = c->arena_bytes; h.arena_ptr = (uint64_t)(uintptr_t)c->arena;
     const cudaError_t e = cudaIpcGetMemHandle(&h.ipc, c->arena);
     if (e != cudaSuccess) { cudaGetLastError(); memset(&h.ipc, 0, sizeof h.ipc); }     // in-process peers still work without IPC
@@ -1250,9 +1084,9 @@ int meao_band_connect(MeaoCtx *c, int32_t side, const MeaoPeerHandle *peer)
     PeerHandlePod h;
     memcpy(&h, peer->bytes, sizeof h);
     if (h.magic != kPeerMagic) return fail(c, MEAO_ERR_INVALID, "not a MeaoPeerHandle");
-    if (h.W != c->W || h.H != c->H || h.arena_bytes != c->arena_bytes)
+    if (h.W != c->g.W || h.H != c->g.H || h.arena_bytes != c->arena_bytes)
         return fail(c, MEAO_ERR_INVALID, "neighbour frame %dx%d (arena %llu B) differs from this context's %dx%d (%zu B)", h.W, h.H,
-                    (unsigned long long)h.arena_bytes, c->W, c->H, c->arena_bytes);
+                    (unsigned long long)h.arena_bytes, c->g.W, c->g.H, c->arena_bytes);
     if (h.pid == (int64_t)getpid()) {
         if (h.device != c->device) {
             int can = 0;
@@ -1289,8 +1123,8 @@ static int record_exchange(MeaoCtx *c, cudaStream_t s)
         for (int k = 1; k <= 4; k++) {
             const int rows = r[k].hi - r[k].lo;
             if (rows <= 0) continue;
-            const size_t off = (size_t)((char *)(c->low[k] + (size_t)r[k].lo * c->low_pitch[k]) - (char *)c->arena);
-            const size_t bytes = (size_t)rows * c->low_pitch[k] * sizeof(float);          // whole pitched rows: contiguous, 128 B aligned
+            const size_t off = (size_t)((char *)(c->bufs.low[k] + (size_t)r[k].lo * c->g.low_pitch[k]) - (char *)c->arena);
+            const size_t bytes = (size_t)rows * c->g.low_pitch[k] * sizeof(float);          // whole pitched rows: contiguous, 128 B aligned
             XchgSeg &g = a.seg[a.nseg++];
             g.src = (const uint4 *)((char *)c->arena + off);
             g.dst = (uint4 *)((char *)c->peer_base[side] + off);
@@ -1333,9 +1167,9 @@ int meao_band_step_host(MeaoCtx *c, const void *depth_host, int32_t kind, uint8_
     const size_t rows = (size_t)(c->band1 - c->band0);
     cudaStream_t s = c->slot_stream[0];
     const size_t esz = (kind == MEAO_DEPTH_RAW_D16_UNORM) ? 2 : 4;
-    CUDA_TRY(c, cudaMemcpyAsync(c->depth_stage[0], depth_host, rows * c->W * esz, cudaMemcpyHostToDevice, s));
+    CUDA_TRY(c, cudaMemcpyAsync(c->depth_stage[0], depth_host, rows * c->g.W * esz, cudaMemcpyHostToDevice, s));
     if ((rc = meao_band_step(c, c->depth_stage[0], kind, c->ao_stage[0], s))) return rc;
-    CUDA_TRY(c, cudaMemcpyAsync(ao_host, c->ao_stage[0], rows * c->W, cudaMemcpyDeviceToHost, s));
+    CUDA_TRY(c, cudaMemcpyAsync(ao_host, c->ao_stage[0], rows * c->g.W, cudaMemcpyDeviceToHost, s));
     return MEAO_OK;
 }
 
@@ -1384,11 +1218,10 @@ int meao_render_batch(MeaoCtx *c, const void *depth, int32_t kind, int32_t frame
     if (!depth || !ao_out) return fail(c, MEAO_ERR_INVALID, "depth / ao_out is NULL");
     if (kind < MEAO_DEPTH_RAW_F32 || kind > MEAO_DEPTH_RAW_D24S8) return fail(c, MEAO_ERR_INVALID, "bad depth kind %d", kind);
     if (frames < 1 || frames > 65535) return fail(c, MEAO_ERR_INVALID, "frames %d not in 1..65535", frames);
-    if (c->band0 != 0 || c->band1 != c->H) return fail(c, MEAO_ERR_UNSUPPORTED, "batched frames need a whole-frame context (no row band)");
+    if (c->band0 != 0 || c->band1 != c->g.H) return fail(c, MEAO_ERR_UNSUPPORTED, "batched frames need a whole-frame context (no row band)");
     if ((rc = reserve_batch(c, frames))) return rc;
     cudaStream_t s = (cudaStream_t)stream;
-    const size_t esz = (kind == MEAO_DEPTH_RAW_D16_UNORM) ? 2 : 4;
-    const BatchRun run{frames, (long long)c->W * c->H * (long long)esz};
+    const BatchRun run{frames, (long long)c->g.W * c->g.H * depth_elem_bytes(depth_in_format(kind)), (long long)c->batch.slot_bytes};
     c->batch.last_frames = frames;
     if (c->flags & MEAO_FLAG_NO_GRAPH) return record_frame(c, depth, kind, ao_out, s, false, &run);
     // one graph replay for the whole batch: the DAG of record_frame_dag, every node covering all frames
@@ -1402,37 +1235,15 @@ int meao_render_batch(MeaoCtx *c, const void *depth, int32_t kind, int32_t frame
 int meao_get_batch_buffer(MeaoCtx *c, int32_t frame, int32_t id, void *host_out, size_t host_bytes)
 {
     int rc = ensure_ready(c); if (rc) return rc;
-    int lvl, slices, elem;
-    if (!host_out || id == MEAO_BUF_AMBIENT_OCCLUSION || buffer_info(c, id, &lvl, &slices, &elem))
-        return fail(c, MEAO_ERR_INVALID, "bad batch buffer id %d (the AO of a batch is in the caller's buffer)", id);
     const BatchArena &b = c->batch;
+    BufferView v;
+    if (!host_out || id == MEAO_BUF_AMBIENT_OCCLUSION || !buffer_view(c->g, b.bufs, nullptr, id, &v))
+        return fail(c, MEAO_ERR_INVALID, "bad batch buffer id %d (the AO of a batch is in the caller's buffer)", id);
     if (frame < 0 || frame >= b.last_frames) return fail(c, MEAO_ERR_INVALID, "frame %d not in the last batch (%d frames)", frame, b.last_frames);
-    const size_t need = (size_t)c->lw[lvl] * c->lh[lvl] * slices * elem;
-    if (host_bytes < need) return fail(c, MEAO_ERR_INVALID, "buffer %d needs %zu bytes, got %zu", id, need, host_bytes);
+    if (host_bytes < v.bytes()) return fail(c, MEAO_ERR_INVALID, "buffer %d needs %zu bytes, got %zu", id, v.bytes(), host_bytes);
     CUDA_TRY(c, cudaDeviceSynchronize());     // debug path: batches may be in flight on any caller stream
-    const size_t fo = (size_t)frame * b.slot_bytes;
-    if (slices == 16) {
-        const int k = id - 5;
-        __half *tmp = nullptr;
-        CUDA_TRY(c, cudaMalloc(&tmp, need));
-        const float pad = host_f16_round((b.last_kind != MEAO_DEPTH_LINEAR_F32) ? c->plan.pad[k] : 0.0f);
-        cudaError_t e = launch_synth_tiled((const float *)((const char *)b.low[k] + fo), c->lw[k], c->lh[k], c->low_pitch[k], c->lw[k + 2], c->lh[k + 2], pad, tmp, c->stream);
-        if (e == cudaSuccess) e = cudaMemcpyAsync(host_out, tmp, need, cudaMemcpyDeviceToHost, c->stream);
-        if (e == cudaSuccess) e = cudaStreamSynchronize(c->stream);
-        cudaFree(tmp);
-        if (e != cudaSuccess) return fail(c, MEAO_ERR_CUDA, "tiled view: %s", cudaGetErrorString(e));
-        return MEAO_OK;
-    }
-    const void *p; size_t pitch;
-    if (id == 1) { p = b.lin; pitch = (size_t)c->lin_pitch * 2; }
-    else if (id >= 2 && id <= 5) { p = b.low[id - 1]; pitch = (size_t)c->low_pitch[id - 1] * 4; }
-    else if (id >= 10 && id <= 13) { p = b.occ[id - 9]; pitch = c->occ_pitch[id - 9]; }
-    else if (id >= 14 && id <= 16) { p = b.comb[id - 13]; pitch = c->occ_pitch[id - 13]; }
-    else { p = b.hq[id - 17]; pitch = c->occ_pitch[id - 17]; }
-    const size_t wb = (size_t)c->lw[lvl] * elem;
-    CUDA_TRY(c, cudaMemcpy2DAsync(host_out, wb, (const char *)p + fo, pitch, wb, c->lh[lvl], cudaMemcpyDeviceToHost, c->stream));
-    CUDA_TRY(c, cudaStreamSynchronize(c->stream));
-    return MEAO_OK;
+    v.ptr = (char *)v.ptr + (size_t)frame * b.slot_bytes;
+    return transfer_view(c, v, b.last_kind, host_out, true);
 }
 
 int meao_render_host_async(MeaoCtx *c, const void *depth_host, int32_t kind, uint8_t *ao_host, int32_t slot)
@@ -1443,13 +1254,13 @@ int meao_render_host_async(MeaoCtx *c, const void *depth_host, int32_t kind, uin
     const size_t rows = (size_t)(c->band1 - c->band0);
     cudaStream_t s = c->slot_stream[slot];
     const size_t esz = (kind == MEAO_DEPTH_RAW_D16_UNORM) ? 2 : 4;
-    CUDA_TRY(c, cudaMemcpyAsync(c->depth_stage[slot], depth_host, rows * c->W * esz, cudaMemcpyHostToDevice, s));
+    CUDA_TRY(c, cudaMemcpyAsync(c->depth_stage[slot], depth_host, rows * c->g.W * esz, cudaMemcpyHostToDevice, s));
     // the two slots share the context's intermediates: kernels of consecutive frames are serialised, copies are not
     if (c->compute_done_valid) CUDA_TRY(c, cudaStreamWaitEvent(s, c->compute_done, 0));
     if ((rc = meao_render(c, c->depth_stage[slot], kind, c->ao_stage[slot], s))) return rc;
     CUDA_TRY(c, cudaEventRecord(c->compute_done, s));
     c->compute_done_valid = true;
-    CUDA_TRY(c, cudaMemcpyAsync(ao_host, c->ao_stage[slot], rows * c->W, cudaMemcpyDeviceToHost, s));
+    CUDA_TRY(c, cudaMemcpyAsync(ao_host, c->ao_stage[slot], rows * c->g.W, cudaMemcpyDeviceToHost, s));
     CUDA_TRY(c, cudaEventRecord(c->slot_done[slot], s));
     return MEAO_OK;
 }
@@ -1518,74 +1329,33 @@ int meao_stage_upsample(MeaoCtx *c, int32_t lo_level, void *ao_out, void *stream
 
 int meao_buffer_desc(const MeaoCtx *c, int32_t id, MeaoBufferDesc *out)
 {
-    if (!c || !out || c->W <= 0) return MEAO_ERR_INVALID;
-    int lvl, slices, elem;
-    if (buffer_info(c, id, &lvl, &slices, &elem)) return MEAO_ERR_INVALID;
-    out->width = c->lw[lvl]; out->height = c->lh[lvl]; out->slices = slices; out->elem_bytes = elem;
+    if (!c || !out || c->g.W <= 0) return MEAO_ERR_INVALID;
+    BufferView v;
+    if (!buffer_view(c->g, c->bufs, c->result, id, &v)) return MEAO_ERR_INVALID;
+    out->width = v.w; out->height = v.h; out->slices = v.slices; out->elem_bytes = v.elem;
     return MEAO_OK;
 }
 
 int meao_get_buffer(MeaoCtx *c, int32_t id, void *host_out, size_t host_bytes)
 {
     int rc = ensure_ready(c); if (rc) return rc;
-    int lvl, slices, elem;
-    if (!host_out || buffer_info(c, id, &lvl, &slices, &elem)) return fail(c, MEAO_ERR_INVALID, "bad buffer id %d", id);
-    const size_t need = (size_t)c->lw[lvl] * c->lh[lvl] * slices * elem;
-    if (host_bytes < need) return fail(c, MEAO_ERR_INVALID, "buffer %d needs %zu bytes, got %zu", id, need, host_bytes);
+    BufferView v;
+    if (!host_out || !buffer_view(c->g, c->bufs, c->result, id, &v)) return fail(c, MEAO_ERR_INVALID, "bad buffer id %d", id);
+    if (host_bytes < v.bytes()) return fail(c, MEAO_ERR_INVALID, "buffer %d needs %zu bytes, got %zu", id, v.bytes(), host_bytes);
     CUDA_TRY(c, cudaDeviceSynchronize());     // debug path: frames may be in flight on any caller stream
-    if (slices == 16) {
-        const int k = id - 5;
-        __half *tmp = nullptr;
-        CUDA_TRY(c, cudaMalloc(&tmp, need));
-        const float pad = host_f16_round((c->last_kind != MEAO_DEPTH_LINEAR_F32) ? c->plan.pad[k] : 0.0f);
-        cudaError_t e = launch_synth_tiled(c->low[k], c->lw[k], c->lh[k], c->low_pitch[k], c->lw[k + 2], c->lh[k + 2], pad, tmp, c->stream);
-        if (e == cudaSuccess) e = cudaMemcpyAsync(host_out, tmp, need, cudaMemcpyDeviceToHost, c->stream);
-        if (e == cudaSuccess) e = cudaStreamSynchronize(c->stream);
-        cudaFree(tmp);
-        if (e != cudaSuccess) return fail(c, MEAO_ERR_CUDA, "tiled view: %s", cudaGetErrorString(e));
-        return MEAO_OK;
-    }
-    void *p; size_t pitch;
-    buffer_ptr(c, id, &p, &pitch);
-    const size_t wb = (size_t)c->lw[lvl] * elem;
-    if (id == MEAO_BUF_AMBIENT_OCCLUSION && c->last_out) {
-        // the last frame wrote the AO texture straight into the caller's buffer; regenerate the debug view
-        // from the (still resident) Combined1 / LowDepth1 / LinearDepth with the same kernel
-        const int64_t before = c->launches;
-        if ((rc = record_upsample(c, 1, nullptr, c->stream))) return rc;
-        c->launches = before;
-    }
-    CUDA_TRY(c, cudaMemcpy2DAsync(host_out, wb, p, pitch, wb, c->lh[lvl], cudaMemcpyDeviceToHost, c->stream));
-    CUDA_TRY(c, cudaStreamSynchronize(c->stream));
-    return MEAO_OK;
+    if (id == MEAO_BUF_AMBIENT_OCCLUSION && (rc = refresh_result(c, c->stream))) return rc;
+    return transfer_view(c, v, c->last_kind, host_out, true);
 }
 
 int meao_debug_view(MeaoCtx *c, int32_t id, void *out, void *stream)
 {
     int rc = ensure_ready(c); if (rc) return rc;
-    int lvl, slices, elem;
-    if (!out || buffer_info(c, id, &lvl, &slices, &elem)) return fail(c, MEAO_ERR_INVALID, "bad buffer id %d / out is NULL", id);
-    if (c->band0 != 0 || c->band1 != c->H) return fail(c, MEAO_ERR_UNSUPPORTED, "debug views need a whole-frame context (no row band)");
+    BufferView v;
+    if (!out || !buffer_view(c->g, c->bufs, c->result, id, &v)) return fail(c, MEAO_ERR_INVALID, "bad buffer id %d / out is NULL", id);
+    if (c->band0 != 0 || c->band1 != c->g.H) return fail(c, MEAO_ERR_UNSUPPORTED, "debug views need a whole-frame context (no row band)");
     cudaStream_t s = (cudaStream_t)stream;
-    DebugViewArgs a{};
-    a.W = c->W; a.H = c->H; a.out = (uint8_t *)out; a.out_pitch = c->W;
-    if (slices == 16) {                                             // AO.cs:810-814: Blit.shader pass 4
-        const int k = id - 5;
-        a.tiled = 1; a.src = c->low[k]; a.elem = 4; a.spitch = c->low_pitch[k];
-        a.sw = c->lw[k + 2]; a.sh = c->lh[k + 2]; a.lw = c->lw[k]; a.lh = c->lh[k];
-        a.pad = host_f16_round((c->last_kind != MEAO_DEPTH_LINEAR_F32) ? c->plan.pad[k] : 0.0f);
-    } else {                                                        // AO.cs:815-819
-        if (id == MEAO_BUF_AMBIENT_OCCLUSION && c->last_out) {
-            // the last frame wrote the AO texture straight into the caller's buffer: regenerate the context's own copy
-            const int64_t before = c->launches;
-            if ((rc = record_upsample(c, 1, nullptr, s))) return rc;
-            c->launches = before;
-        }
-        void *p; size_t pitch;
-        buffer_ptr(c, id, &p, &pitch);
-        a.src = p; a.elem = elem; a.spitch = (int)(pitch / elem); a.sw = c->lw[lvl]; a.sh = c->lh[lvl];
-    }
-    CUDA_TRY(c, launch_debug_view(a, s));
+    if (id == MEAO_BUF_AMBIENT_OCCLUSION && (rc = refresh_result(c, s))) return rc;
+    CUDA_TRY(c, launch_debug_view(debug_view_args(c->g, c->plan, v, c->last_kind != MEAO_DEPTH_LINEAR_F32, (uint8_t *)out), s));
     c->launches++;
     return MEAO_OK;
 }
@@ -1593,24 +1363,18 @@ int meao_debug_view(MeaoCtx *c, int32_t id, void *out, void *stream)
 int meao_set_buffer(MeaoCtx *c, int32_t id, const void *host_in, size_t host_bytes)
 {
     int rc = ensure_ready(c); if (rc) return rc;
-    int lvl, slices, elem;
-    if (!host_in || buffer_info(c, id, &lvl, &slices, &elem) || slices != 1)
+    BufferView v;
+    if (!host_in || !buffer_view(c->g, c->bufs, c->result, id, &v) || v.slices != 1)
         return fail(c, MEAO_ERR_INVALID, "buffer id %d cannot be set", id);
-    const size_t need = (size_t)c->lw[lvl] * c->lh[lvl] * elem;
-    if (host_bytes < need) return fail(c, MEAO_ERR_INVALID, "buffer %d needs %zu bytes, got %zu", id, need, host_bytes);
-    void *p; size_t pitch;
-    buffer_ptr(c, id, &p, &pitch);
-    const size_t wb = (size_t)c->lw[lvl] * elem;
+    if (host_bytes < v.bytes()) return fail(c, MEAO_ERR_INVALID, "buffer %d needs %zu bytes, got %zu", id, v.bytes(), host_bytes);
     CUDA_TRY(c, cudaDeviceSynchronize());
-    CUDA_TRY(c, cudaMemcpy2DAsync(p, pitch, host_in, wb, wb, c->lh[lvl], cudaMemcpyHostToDevice, c->stream));
-    CUDA_TRY(c, cudaStreamSynchronize(c->stream));
-    return MEAO_OK;
+    return transfer_view(c, v, c->last_kind, (void *)host_in, false);
 }
 
 // The constant getters work without a device context being current: they only need the plan.
 static int plan_only(MeaoCtx *c)
 {
-    if (!c || c->W <= 0) return MEAO_ERR_INVALID;
+    if (!c || c->g.W <= 0) return MEAO_ERR_INVALID;
     if (c->plan_dirty) { build_plan(c); c->graphs_stale = true; }    // the captured graphs are dropped by the next ensure_ready, on c->device
     return 0;
 }
@@ -1664,7 +1428,7 @@ int meao_composite_framebuffer(MeaoCtx *c, const void *ao, void *color, int32_t 
 {
     int rc = ensure_ready(c); if (rc) return rc;
     if ((rc = composite_args(c, ao, color, fmt))) return rc;
-    const long long npix = (long long)c->W * (c->band1 - c->band0);
+    const long long npix = (long long)c->g.W * (c->band1 - c->band0);
     CUDA_TRY(c, launch_composite((const uint8_t *)ao, color, npix, fmt == MEAO_FMT_RGBA16_FLOAT, 1, 1, 0, (cudaStream_t)stream));
     c->launches++;
     return MEAO_OK;
@@ -1674,7 +1438,7 @@ int meao_composite_gbuffer(MeaoCtx *c, const void *ao, void *g0, void *g3, int32
 {
     int rc = ensure_ready(c); if (rc) return rc;
     if ((rc = composite_args(c, ao, g0, MEAO_FMT_RGBA8_UNORM)) || (rc = composite_args(c, ao, g3, fmt3))) return rc;
-    const long long npix = (long long)c->W * (c->band1 - c->band0);
+    const long long npix = (long long)c->g.W * (c->band1 - c->band0);
     CUDA_TRY(c, launch_composite((const uint8_t *)ao, g0, npix, 0, 0, 1, 1, (cudaStream_t)stream));                               // gbuffer0.a
     CUDA_TRY(c, launch_composite((const uint8_t *)ao, g3, npix, fmt3 == MEAO_FMT_RGBA16_FLOAT, 1, 0, 1, (cudaStream_t)stream));   // gbuffer3.rgb
     c->launches += 2;
@@ -1685,7 +1449,7 @@ int meao_composite_debug(MeaoCtx *c, const void *view, void *color, int32_t fmt,
 {
     int rc = ensure_ready(c); if (rc) return rc;
     if ((rc = composite_args(c, view, color, fmt))) return rc;
-    const long long npix = (long long)c->W * (c->band1 - c->band0);
+    const long long npix = (long long)c->g.W * (c->band1 - c->band0);
     CUDA_TRY(c, launch_debug_composite((const uint8_t *)view, color, npix, fmt == MEAO_FMT_RGBA16_FLOAT, (cudaStream_t)stream));
     c->launches++;
     return MEAO_OK;
@@ -1720,14 +1484,14 @@ int meao_kernels_per_frame(const MeaoCtx *c)
 {
     if (c && c->variants.single_scale) return 3;      // Downsample1 + Render level 1 + the final-style Upsample
     int n = 9;
-    if (c) for (int k = 1; k <= 4; k++) n += hq_level(c, k) ? 1 : 0;
+    if (c) for (int k = 1; k <= 4; k++) n += hq_level(c->variants, k) ? 1 : 0;
     return n;
 }
 
 int64_t meao_algorithmic_bytes(const MeaoCtx *c, int32_t stage)
 {
-    if (!c || c->W <= 0) return MEAO_ERR_INVALID;
-    auto px = [&](int l) { return (int64_t)c->lw[l] * c->lh[l]; };
+    if (!c || c->g.W <= 0) return MEAO_ERR_INVALID;
+    auto px = [&](int l) { return (int64_t)c->g.lw[l] * c->g.lh[l]; };
     // SURVEY.md 8(d): every buffer of the reference data-flow read once per consuming stage, written once
     const int64_t ds1 = 6 * px(0) + 4 * px(1) + 4 * px(2) + 32 * px(3) + 32 * px(4);
     const int64_t ds2 = 4 * px(2) + 4 * px(3) + 4 * px(4) + 32 * px(5) + 32 * px(6);

@@ -1,49 +1,109 @@
 // emu_driver.cpp -- runs one frame through the HOST-compiled kernel sources (TEST INFRASTRUCTURE ONLY, see cuda_emu.h).
-// It owns pitched buffers laid out like MeaoCtx's arena and fills PrepareArgs / RenderArgs / UpsampleArgs the way
-// meao_api.cu's record_downsample / record_render / record_upsample do; the per-dispatch constants are handed in by the
-// test (which reads them from a plan-only libmeao context), so the planner itself is not duplicated here.
+// It lays out one frame slot and builds every argument block and TMA map with libmeao's own host logic
+// (miniengineao_b200/csrc/frame_plan.h); the per-dispatch constants are handed in by the test (which reads them from a
+// plan-only libmeao context), so the planner itself is not duplicated here.  tests/emu_batch compiles this file with the
+// 3-D TMA emulation and drives the same functions over a batch arena.
 #include <cstdlib>
 #include <cstring>
 #include <vector>
 
 #include "../../miniengineao_b200/csrc/common.cuh"
 #include "../../miniengineao_b200/csrc/kernels.h"
+#include "../../miniengineao_b200/csrc/frame_plan.h"
 
 using namespace meao;
 
 namespace {
 
-inline int align_up(int x, int a) { return (x + a - 1) / a * a; }
 template <class T> T *alloc(size_t n) { void *p = nullptr; if (posix_memalign(&p, 256, (n * sizeof(T) + 255) / 256 * 256 + 256)) abort(); memset(p, 0, n * sizeof(T)); return (T *)p; }
 
+// The buffers a launch works in: the frame's own slot, or slot 0 of a batch (batch != nullptr, tests/emu_batch only).
+struct EmuArena { FrameBufs bufs; uint32_t *tile_ctr; const BatchRun *batch; };
+
 struct Emu {
-    int W, H, lw[7], lh[7];
-    __half *lin; int lin_pitch;
-    float *low[5]; int low_pitch[5];
-    uint8_t *occ[5], *comb[4], *hq[5]; int occ_pitch[5];
-    uint8_t *result; int result_pitch;
+    FrameGeom g;
+    char *slot = nullptr;                   // one frame slot (SlotLayout)
+    uint8_t *result = nullptr;
+    uint32_t tile_ctr[8] = {0, 0, 0, 0, 0, 0, 0, 0};   // persistent blur_upsample grid: tile cursor + finished-CTA count per level
+    EmuArena arena{};                       // the slot, its counters
     // constants (set by emu_set_constants)
-    float zbx = 0, zby = 1; int raw = 1, reversed_z = 1;
-    float inv_thickness[5][12], inv_thickness_wide[5][12], sample_weight[5][12];
-    float reject_fadeoff = -1, intensity = 1, pad[5] = {0, 0, 0, 0, 0};
-    float nfs[5], step[5], kblur[5], tol[5];
-    int hq_mask = 0, exhaustive = 0;
+    Plan plan{};
+    MeaoVariants v = {0, 0, 0, 0};
+    int raw = 1, reversed_z = 1;
     int use_tma = 1;        // 1: interior tiles take the kernels' TMA path (emulated box loads), 0: every tile gathers
     // row band (meao_set_row_band): rows of level k to PRODUCE, k = 0..4 (meao_band_rows "produce"); default = whole frame
-    int band0 = 0, band1 = 0, need_lo[5] = {0, 0, 0, 0, 0}, need_hi[5] = {0, 0, 0, 0, 0};
-    int ren_tile = -1;      // render tile-height variant (index into kRenderTileHs); -1 = the planner's rule (meao_api.cu render_tile_variant)
-    int single_scale = 0;   // MeaoVariants.single_scale
-    uint32_t tile_ctr[8] = {0, 0, 0, 0, 0, 0, 0, 0};   // persistent blur_upsample grid: tile cursor + finished-CTA count per level
+    Range band{0, 0}, need[5] = {};
+    int ren_tile = -1;      // render tile-height variant (index into kRenderTileHs); -1 = the planner's rule (render_tile_variant)
     BandFlags flags{};      // native neighbour exchange (band_exchange.cu)
     uint32_t host_error = 0;
 };
 
-// what MeaoCtx::make_map hands to cuTensorMapEncodeTiled
-CUtensorMap make_map(const void *base, int elem, int w, int h, int pitch_elems, int bw, int bh)
+// what libmeao's encode_map hands to cuTensorMapEncodeTiled; a batch: the 3-D map of tests/emu_batch/cuda_emu_3d.h
+CUtensorMap emu_map(const MapSpec &s, const BatchRun *batch = nullptr)
 {
     CUtensorMap m{};
-    m.base = base; m.elem = elem; m.w = w; m.h = h; m.pitch_bytes = (size_t)pitch_elems * elem; m.bw = bw; m.bh = bh;
+    m.base = s.base; m.elem = s.elem; m.w = s.w; m.h = s.h; m.pitch_bytes = s.pitch_bytes; m.bw = s.bw; m.bh = s.bh;
+    if (batch) { m.pad_[0] = (uint64_t)batch->frames; m.pad_[1] = (uint64_t)batch->slot_bytes; }
     return m;
+}
+
+// The three recorders of meao_api.cu; the batch launchers exist only in the tests/emu_batch build.
+void run_downsample(Emu *e, const EmuArena &ar, const void *depth, int in_format)
+{
+    const PrepareArgs a = prepare_args(e->g, ar.bufs, e->plan, depth, in_format, e->raw != 0, e->reversed_z, e->band, ar.batch);
+#ifdef MEAO_EMU_TMA_3D
+    if (ar.batch) { launch_prepare_depth_batch(PrepareBatchArgs{a, ar.batch->in_frame_bytes, ar.batch->slot_bytes}, ar.batch->frames, nullptr); return; }
+#endif
+    launch_prepare_depth(a, nullptr);
+}
+
+void run_render(Emu *e, const EmuArena &ar, int k, bool wide)
+{
+    const int frames = ar.batch ? ar.batch->frames : 1;
+    const int tv = e->ren_tile >= 0 ? e->ren_tile : render_tile_variant(e->g.lw[k], e->need[k], frames);
+    const RenderArgs a = render_args(e->g, ar.bufs, e->plan, k, wide, e->v.sample_exhaustively != 0, e->raw != 0, e->need[k], tv);
+    const CUtensorMap m = emu_map(render_map(e->g, ar.bufs, k, tv, wide), ar.batch);
+#ifdef MEAO_EMU_TMA_3D
+    if (ar.batch) { launch_render_ao_batch(m, e->use_tma != 0, RenderBatchArgs{a, ar.batch->slot_bytes}, frames, nullptr); return; }
+#endif
+    launch_render_ao(m, e->use_tma != 0, a, nullptr);
+}
+
+void run_upsample(Emu *e, const EmuArena &ar, int lo, uint8_t *ao_out)
+{
+    const UpsamplePreminArgs pa = upsample_args(e->g, ar.bufs, e->plan, e->v, lo, e->need[lo - 1], ao_out, e->result, e->band.lo,
+                                                ar.tile_ctr, ar.batch);
+    const CUtensorMap md = emu_map(ups_depth_map(e->g, ar.bufs, lo), ar.batch);
+    const CUtensorMap ma = emu_map(ups_ao_map(e->g, pa.base.lo_ao, lo), ar.batch);
+    const CUtensorMap mh = emu_map(ups_ao_map(e->g, ar.bufs.hq[lo], lo), ar.batch);
+#ifdef MEAO_EMU_TMA_3D
+    if (ar.batch) {
+        const UpsampleBatchArgs ba{pa, ar.batch->slot_bytes, ups_out_frame_bytes(e->g, lo, *ar.batch), ar.batch->frames, 0};
+        launch_blur_upsample_batch(md, ma, &mh, e->use_tma != 0, ba, nullptr);
+        return;
+    }
+#endif
+    launch_blur_upsample(md, ma, &mh, e->use_tma != 0, pa.base, pa.lo_ao2, pa.lo_a2pitch, nullptr);
+}
+
+// everything after the downsample, in meao_api.cu's record_frame order; ao_out = nullptr: the AO texture
+void run_renders_upsamples(Emu *e, const EmuArena &ar, uint8_t *ao_out)
+{
+    const int kmax = e->v.single_scale ? 1 : 4;       // single-scale: Render level 1 + the final-style Upsample only
+    for (int k = 1; k <= kmax; k++) run_render(e, ar, k, false);
+    for (int k = 1; k <= kmax; k++) if (hq_level(e->v, k)) run_render(e, ar, k, true);
+    for (int lo = kmax; lo >= 1; lo--) run_upsample(e, ar, lo, lo == 1 ? ao_out : nullptr);
+}
+
+// a buffer view in the reference layout / native type (meao_get_buffer)
+void read_view(const Emu *e, const BufferView &v, void *out)
+{
+    if (v.slices == 16) {
+        const int k = v.level;
+        launch_synth_tiled((const float *)v.ptr, e->g.lw[k], e->g.lh[k], e->g.low_pitch[k], v.w, v.h, atlas_pad(e->plan, k, e->raw != 0), (__half *)out, nullptr);
+        return;
+    }
+    for (int y = 0; y < v.h; y++) memcpy((char *)out + (size_t)y * v.w * v.elem, (const char *)v.ptr + (size_t)y * v.pitch_bytes, (size_t)v.w * v.elem);
 }
 
 }  // namespace
@@ -53,27 +113,20 @@ extern "C" {
 void *emu_create(int W, int H)
 {
     Emu *e = new Emu();
-    e->W = W; e->H = H;
-    for (int l = 0; l < 7; l++) { const int d = 1 << l; e->lw[l] = (W + d - 1) / d; e->lh[l] = (H + d - 1) / d; }
-    e->lin_pitch = align_up(W, 64); e->lin = alloc<__half>((size_t)e->lin_pitch * H);
-    e->result_pitch = align_up(W, 128); e->result = alloc<uint8_t>((size_t)e->result_pitch * H);
-    for (int k = 1; k <= 4; k++) {
-        e->low_pitch[k] = align_up(e->lw[k], 32); e->occ_pitch[k] = align_up(e->lw[k], 128);
-        e->low[k] = alloc<float>((size_t)e->low_pitch[k] * e->lh[k]);
-        e->occ[k] = alloc<uint8_t>((size_t)e->occ_pitch[k] * e->lh[k]);
-        e->hq[k] = alloc<uint8_t>((size_t)e->occ_pitch[k] * e->lh[k]);
-        if (k <= 3) e->comb[k] = alloc<uint8_t>((size_t)e->occ_pitch[k] * e->lh[k]);
-    }
-    e->band0 = 0; e->band1 = H;
-    for (int k = 0; k <= 4; k++) { e->need_lo[k] = 0; e->need_hi[k] = e->lh[k]; }
+    e->g = frame_geom(W, H);
+    const SlotLayout s = slot_layout(e->g);
+    e->slot = alloc<char>(s.slot_bytes);
+    e->result = alloc<uint8_t>((size_t)e->g.result_pitch * H);
+    e->arena = EmuArena{frame_bufs(e->slot, s), e->tile_ctr, nullptr};
+    e->band = Range{0, H};
+    for (int k = 0; k <= 4; k++) e->need[k] = Range{0, e->g.lh[k]};
     return e;
 }
 
 void emu_destroy(void *h)
 {
     Emu *e = (Emu *)h;
-    free(e->lin); free(e->result);
-    for (int k = 1; k <= 4; k++) { free(e->low[k]); free(e->occ[k]); free(e->hq[k]); if (k <= 3) free(e->comb[k]); }
+    free(e->slot); free(e->result);
     delete e;
 }
 
@@ -83,84 +136,25 @@ void emu_set_constants(void *h, const float *rc, const float *rcw, const float *
                        int raw, int reversed_z, int hq_mask, int exhaustive)
 {
     Emu *e = (Emu *)h;
+    Plan &p = e->plan;
     for (int k = 1; k <= 4; k++) {
-        memcpy(e->inv_thickness[k], rc + 28 * (k - 1), 48);
-        memcpy(e->sample_weight[k], rc + 28 * (k - 1) + 12, 48);
-        memcpy(e->inv_thickness_wide[k], rcw + 28 * (k - 1), 48);
-        e->pad[k] = (k <= 2) ? pad12 : 0.0f;
+        memcpy(p.inv_thickness[k], rc + 28 * (k - 1), 48);
+        memcpy(p.sample_weight[k], rc + 28 * (k - 1) + 12, 48);
+        memcpy(p.inv_thickness_wide[k], rcw + 28 * (k - 1), 48);
+        p.pad[k] = (k <= 2) ? pad12 : 0.0f;
         const float *u = uc + 8 * (k - 1);
-        e->nfs[k] = u[4]; e->step[k] = u[5]; e->kblur[k] = u[6]; e->tol[k] = u[7];
+        p.noise_filter_strength[k] = u[4]; p.step_size[k] = u[5]; p.blur_tolerance[k] = u[6]; p.upsample_tolerance[k] = u[7];
     }
-    e->reject_fadeoff = rc[26]; e->intensity = rc[27];
-    e->zbx = zb[0]; e->zby = zb[1]; e->raw = raw; e->reversed_z = reversed_z; e->hq_mask = hq_mask; e->exhaustive = exhaustive;
-}
-
-static void run_downsample(Emu *e, const void *depth, int in_format)
-{
-    PrepareArgs a{};
-    a.depth = depth; a.in_format = in_format; a.W = e->W; a.H = e->H; a.depth_row0 = e->band0; a.row0 = e->band0; a.row1 = e->band1;
-    a.lin = e->lin; a.lin_pitch = e->lin_pitch;
-    for (int k = 1; k <= 4; k++) { a.low[k - 1] = e->low[k]; a.low_pitch[k - 1] = e->low_pitch[k]; }
-    a.zbx = e->zbx; a.zby = e->zby; a.raw = e->raw; a.reversed_z = e->reversed_z;
-    a.vec_ok = (((uintptr_t)depth & 15) == 0) && (e->W % (in_format == 1 ? 8 : 4) == 0);
-    launch_prepare_depth(a, nullptr);
-}
-
-static void run_render(Emu *e, int k, bool wide)
-{
-    static const int idx_checker[7] = {1, 3, 4, 8, 11, 6, 10}, idx_exh[12] = {0, 1, 2, 3, 4, 8, 11, 5, 6, 7, 9, 10};
-    const int n = e->exhaustive ? 12 : 7; const int *idx = e->exhaustive ? idx_exh : idx_checker;
-    RenderArgs a{};
-    a.low = e->low[k]; a.lw = e->lw[k]; a.lh = e->lh[k]; a.lpitch = e->low_pitch[k];
-    a.occ = wide ? e->hq[k] : e->occ[k]; a.opitch = e->occ_pitch[k];
-    a.sw = e->lw[k + 2]; a.sh = e->lh[k + 2];
-    a.pad = __half2float(__float2half_rn(e->pad[k]));
-    const float *it = wide ? e->inv_thickness_wide[k] : e->inv_thickness[k];
-    for (int i = 0; i < n; i++) { a.inv_thickness[i] = it[idx[i]]; a.neg_front[i] = -(a.inv_thickness[i] - 0.5f); a.weight[i] = e->sample_weight[k][idx[i]]; }
-    a.reject_fadeoff = e->reject_fadeoff; a.intensity = e->intensity;
-    a.row0 = e->need_lo[k]; a.row1 = e->need_hi[k]; a.wide = wide; a.exhaustive = e->exhaustive;
-    int tv = e->ren_tile;
-    if (tv < 0) {           // meao_api.cu render_tile_variant
-        const int rows = a.row1 - (a.row0 & ~3);
-        for (tv = 0; tv < kRenderTileVariants - 1; tv++)
-            if (((e->lw[k] + 63) / 64) * ((rows + kRenderTileHs[tv] - 1) / kRenderTileHs[tv]) >= 148) break;
-    }
-    a.tile_h = kRenderTileHs[tv];
-    const CUtensorMap map = make_map(e->low[k], 4, e->lw[k], e->lh[k], e->low_pitch[k], wide ? kRenderWideBoxW : kRenderBoxW, render_box_h(a.tile_h, wide));
-    launch_render_ao(map, e->use_tma != 0, a, nullptr);
-}
-
-static void run_upsample(Emu *e, int lo)
-{
-    const int hi = lo - 1;
-    UpsampleArgs a{};
-    a.lo_depth = e->low[lo]; a.low = e->lw[lo]; a.loh = e->lh[lo]; a.lo_dpitch = e->low_pitch[lo];
-    a.lo_ao = (e->single_scale && lo == 1) ? e->occ[1] : (lo == 4) ? e->occ[4] : e->comb[lo]; a.lo_apitch = e->occ_pitch[lo];
-    if (hi == 0) { a.hi_depth = e->lin; a.hi_is_half = 1; a.hi_dpitch = e->lin_pitch; a.hi_ao = nullptr; a.out = e->result; a.out_pitch = e->result_pitch; }
-    else { a.hi_depth = e->low[hi]; a.hi_is_half = 0; a.hi_dpitch = e->low_pitch[hi]; a.hi_ao = e->occ[hi]; a.hi_apitch = e->occ_pitch[hi]; a.out = e->comb[hi]; a.out_pitch = e->occ_pitch[hi]; }
-    a.out_row_origin = 0; a.out_vec_ok = 1;
-    a.hiw = e->lw[hi]; a.hih = e->lh[hi];
-    a.noise_filter_strength = e->nfs[lo]; a.step_size = e->step[lo]; a.blur_tolerance = e->kblur[lo]; a.upsample_tolerance = e->tol[lo];
-    auto safe = [](float x) { return x >= 8.673617379884035e-19f && x < 1152921504606846976.0f; };
-    a.fast_div_ok = safe(a.upsample_tolerance) && safe(a.noise_filter_strength);
-#if MEAO_UPS_STATIC_GUARD || MEAO_UPS_V2
-    a.fast_div_ok = a.fast_div_ok && a.upsample_tolerance >= 2.7755575615628914e-17f && a.noise_filter_strength >= 2.220446049250313e-16f &&
-                    a.noise_filter_strength < 288230376151711744.0f;
-#endif
-    a.row0 = e->need_lo[hi]; a.row1 = e->need_hi[hi];
-    a.tile_ctr = e->tile_ctr + 2 * (lo - 1);
-    const bool premin = ((e->hq_mask >> (lo - 1)) & 1) != 0;
-    const CUtensorMap md = make_map(e->low[lo], 4, e->lw[lo], e->lh[lo], e->low_pitch[lo], kUpsDepthBoxW, kUpsDepthBoxH);
-    const CUtensorMap ma = make_map(a.lo_ao, 1, e->lw[lo], e->lh[lo], e->occ_pitch[lo], kUpsAoBoxW, kUpsAoBoxH);
-    const CUtensorMap mh = make_map(e->hq[lo], 1, e->lw[lo], e->lh[lo], e->occ_pitch[lo], kUpsAoBoxW, kUpsAoBoxH);
-    launch_blur_upsample(md, ma, &mh, e->use_tma != 0, a, premin ? e->hq[lo] : nullptr, e->occ_pitch[lo], nullptr);
+    p.reject_fadeoff = rc[26]; p.intensity = rc[27];
+    memcpy(p.zb, zb, sizeof p.zb);
+    e->raw = raw; e->reversed_z = reversed_z; e->v.high_quality_mask = hq_mask; e->v.sample_exhaustively = exhaustive;
 }
 
 // aborts (on purpose) with the emulated TMA's alignment complaint: an f32 box starting at x = 3
 int emu_selfcheck_unaligned_tma()
 {
     alignas(128) static float src[64 * 8], dst[16 * 4];
-    const CUtensorMap m = make_map(src, 4, 64, 8, 64, 16, 4);
+    const CUtensorMap m = emu_map(MapSpec{src, 4, 64, 8, 64 * 4, 16, 4});
     meao_emu::tma_load_2d(dst, &m, 3, 0);
     return 0;
 }
@@ -169,17 +163,14 @@ long long emu_tma_box_loads() { return meao_emu::tma_box_loads; }
 
 void emu_set_tma(void *h, int use_tma) { ((Emu *)h)->use_tma = use_tma; }
 void emu_set_render_tile(void *h, int variant) { ((Emu *)h)->ren_tile = variant; }
-void emu_set_single_scale(void *h, int on) { ((Emu *)h)->single_scale = on; }
+void emu_set_single_scale(void *h, int on) { ((Emu *)h)->v.single_scale = on; }
 
 // in_format: 0 = f32, 1 = D16 codes, 2 = D24S8 words (PrepareArgs.in_format); depth must be 16-byte aligned
 void emu_run(void *h, const void *depth, int in_format)
 {
     Emu *e = (Emu *)h;
-    run_downsample(e, depth, in_format);
-    if (e->single_scale) { run_render(e, 1, false); run_upsample(e, 1); return; }    // record_frame_dag, single_scale branch
-    for (int k = 1; k <= 4; k++) run_render(e, k, false);
-    for (int k = 1; k <= 4; k++) if ((e->hq_mask >> (k - 1)) & 1) run_render(e, k, true);
-    for (int lo = 4; lo >= 1; lo--) run_upsample(e, lo);
+    run_downsample(e, e->arena, depth, in_format);
+    run_renders_upsamples(e, e->arena, nullptr);
 }
 
 // ---- native neighbour exchange: band_exchange_kernel with the segments meao_api.cu's record_exchange builds (whole pitched rows
@@ -203,9 +194,9 @@ int emu_band_exchange(void *h, void *up, void *down, const int *rows_up8, const 
             const int lo = rows8[side][2 * (k - 1)], rows = rows8[side][2 * (k - 1) + 1] - lo;
             if (rows <= 0) continue;
             XchgSeg &g = a.seg[a.nseg++];
-            g.src = (const uint4 *)(e->low[k] + (size_t)lo * e->low_pitch[k]);
-            g.dst = (uint4 *)(peer[side]->low[k] + (size_t)lo * e->low_pitch[k]);
-            g.n16 = (uint32_t)((size_t)rows * e->low_pitch[k] * sizeof(float) / 16); g.side = side;
+            g.src = (const uint4 *)(e->arena.bufs.low[k] + (size_t)lo * e->g.low_pitch[k]);
+            g.dst = (uint4 *)(peer[side]->arena.bufs.low[k] + (size_t)lo * e->g.low_pitch[k]);
+            g.n16 = (uint32_t)((size_t)rows * e->g.low_pitch[k] * sizeof(float) / 16); g.side = side;
         }
     }
     launch_band_exchange(a, nullptr);
@@ -227,19 +218,19 @@ void emu_band_flags(void *h, const int *set_ready_ack4, int *out8)
 void emu_set_band(void *h, int row0, int row1, const int *produce10)
 {
     Emu *e = (Emu *)h;
-    e->band0 = row0; e->band1 = row1;
-    for (int k = 0; k <= 4; k++) { e->need_lo[k] = produce10[2 * k]; e->need_hi[k] = produce10[2 * k + 1]; }
+    e->band = Range{row0, row1};
+    for (int k = 0; k <= 4; k++) e->need[k] = Range{produce10[2 * k], produce10[2 * k + 1]};
 }
 
 // every LowDepth texel becomes NaN: rows this band neither produces nor receives must never reach an output
 void emu_poison_low(void *h)
 {
     Emu *e = (Emu *)h;
-    for (int k = 1; k <= 4; k++) for (size_t i = 0; i < (size_t)e->low_pitch[k] * e->lh[k]; i++) e->low[k][i] = __uint_as_float(0x7fc00000u);
+    for (int k = 1; k <= 4; k++) for (size_t i = 0; i < (size_t)e->g.low_pitch[k] * e->g.lh[k]; i++) e->arena.bufs.low[k][i] = __uint_as_float(0x7fc00000u);
 }
 
 // depth_band: the band's rows only (row1 - row0 rows), like meao_render_band_prepare
-void emu_band_phase_a(void *h, const void *depth_band, int in_format) { run_downsample((Emu *)h, depth_band, in_format); }
+void emu_band_phase_a(void *h, const void *depth_band, int in_format) { Emu *e = (Emu *)h; run_downsample(e, e->arena, depth_band, in_format); }
 
 // rows8 = meao_halo_rows(side, send): {lo1,hi1, ..., lo4,hi4}; packed message layout of meao_halo_pack (level 1 first, tight rows)
 void emu_halo(void *h, const int *rows8, float *packed, int pack)
@@ -250,11 +241,11 @@ void emu_halo(void *h, const int *rows8, float *packed, int pack)
     for (int k = 1; k <= 4; k++) {
         const int lo = rows8[2 * (k - 1)], rows = rows8[2 * (k - 1) + 1] - lo;
         if (rows <= 0) continue;
-        float *buf = e->low[k] + (size_t)lo * e->low_pitch[k];
+        float *buf = e->arena.bufs.low[k] + (size_t)lo * e->g.low_pitch[k];
         HaloSeg &g = a.seg[a.nseg++];
-        if (pack) g = HaloSeg{buf, p, e->low_pitch[k], e->lw[k], e->lw[k], rows};
-        else      g = HaloSeg{p, buf, e->lw[k], e->low_pitch[k], e->lw[k], rows};
-        p += (size_t)rows * e->lw[k];
+        if (pack) g = HaloSeg{buf, p, e->g.low_pitch[k], e->g.lw[k], e->g.lw[k], rows};
+        else      g = HaloSeg{p, buf, e->g.lw[k], e->g.low_pitch[k], e->g.lw[k], rows};
+        p += (size_t)rows * e->g.lw[k];
     }
     launch_halo_copy(a, nullptr);
 }
@@ -262,30 +253,16 @@ void emu_halo(void *h, const int *rows8, float *packed, int pack)
 void emu_band_phase_b(void *h)
 {
     Emu *e = (Emu *)h;
-    if (e->single_scale) { run_render(e, 1, false); run_upsample(e, 1); return; }
-    for (int k = 1; k <= 4; k++) run_render(e, k, false);
-    for (int k = 1; k <= 4; k++) if ((e->hq_mask >> (k - 1)) & 1) run_render(e, k, true);
-    for (int lo = 4; lo >= 1; lo--) run_upsample(e, lo);
+    run_renders_upsamples(e, e->arena, nullptr);
 }
 
 // buffer <id> (1..21) in the reference layout / native type, like meao_get_buffer
 int emu_get_buffer(void *h, int id, void *out)
 {
     Emu *e = (Emu *)h;
-    auto copy2d = [&](const void *src, size_t pitch_bytes, int w, int hgt, int elem) {
-        for (int y = 0; y < hgt; y++) memcpy((char *)out + (size_t)y * w * elem, (const char *)src + (size_t)y * pitch_bytes, (size_t)w * elem);
-    };
-    if (id == 1) copy2d(e->lin, (size_t)e->lin_pitch * 2, e->lw[0], e->lh[0], 2);
-    else if (id >= 2 && id <= 5) copy2d(e->low[id - 1], (size_t)e->low_pitch[id - 1] * 4, e->lw[id - 1], e->lh[id - 1], 4);
-    else if (id >= 6 && id <= 9) {
-        const int k = id - 5;
-        launch_synth_tiled(e->low[k], e->lw[k], e->lh[k], e->low_pitch[k], e->lw[k + 2], e->lh[k + 2], __half2float(__float2half_rn(e->pad[k])), (__half *)out, nullptr);
-    }
-    else if (id >= 10 && id <= 13) copy2d(e->occ[id - 9], e->occ_pitch[id - 9], e->lw[id - 9], e->lh[id - 9], 1);
-    else if (id >= 14 && id <= 16) copy2d(e->comb[id - 13], e->occ_pitch[id - 13], e->lw[id - 13], e->lh[id - 13], 1);
-    else if (id == 17) copy2d(e->result, e->result_pitch, e->lw[0], e->lh[0], 1);
-    else if (id >= 18 && id <= 21) copy2d(e->hq[id - 17], e->occ_pitch[id - 17], e->lw[id - 17], e->lh[id - 17], 1);
-    else return -1;
+    BufferView v;
+    if (!buffer_view(e->g, e->arena.bufs, e->result, id, &v)) return -1;
+    read_view(e, v, out);
     return 0;
 }
 
@@ -293,19 +270,9 @@ int emu_get_buffer(void *h, int id, void *out)
 int emu_debug_view(void *h, int id, uint8_t *out)
 {
     Emu *e = (Emu *)h;
-    DebugViewArgs a{};
-    a.W = e->W; a.H = e->H; a.out = out; a.out_pitch = e->W;
-    if (id >= 6 && id <= 9) {
-        const int k = id - 5;
-        a.tiled = 1; a.src = e->low[k]; a.elem = 4; a.spitch = e->low_pitch[k]; a.sw = e->lw[k + 2]; a.sh = e->lh[k + 2]; a.lw = e->lw[k]; a.lh = e->lh[k];
-        a.pad = __half2float(__float2half_rn(e->pad[k]));
-    } else if (id == 1) { a.src = e->lin; a.elem = 2; a.spitch = e->lin_pitch; a.sw = e->lw[0]; a.sh = e->lh[0]; }
-    else if (id >= 2 && id <= 5) { a.src = e->low[id - 1]; a.elem = 4; a.spitch = e->low_pitch[id - 1]; a.sw = e->lw[id - 1]; a.sh = e->lh[id - 1]; }
-    else if (id >= 10 && id <= 13) { a.src = e->occ[id - 9]; a.elem = 1; a.spitch = e->occ_pitch[id - 9]; a.sw = e->lw[id - 9]; a.sh = e->lh[id - 9]; }
-    else if (id >= 14 && id <= 16) { a.src = e->comb[id - 13]; a.elem = 1; a.spitch = e->occ_pitch[id - 13]; a.sw = e->lw[id - 13]; a.sh = e->lh[id - 13]; }
-    else if (id == 17) { a.src = e->result; a.elem = 1; a.spitch = e->result_pitch; a.sw = e->lw[0]; a.sh = e->lh[0]; }
-    else return -1;
-    launch_debug_view(a, nullptr);
+    BufferView v;
+    if (!buffer_view(e->g, e->arena.bufs, e->result, id, &v)) return -1;
+    launch_debug_view(debug_view_args(e->g, e->plan, v, e->raw != 0, out), nullptr);
     return 0;
 }
 
